@@ -8,6 +8,7 @@ QueryPlanPatternDetection.java:106-131, stands behind it in the reference).
 
   python bench.py --gpus N --steps K --warmup W            # the CUDA path (one rank per GPU under torchrun)
   python bench.py --impl reference --gpus N --steps K ...  # the reference's CPU path (oracle port) on host cores
+  python bench.py ... --dump-outputs DIR                   # also write the last timed step's result to DIR/<name>.npy
 
 A step = one /detection request (SaseConnector.evaluate + clearOccurrences == siesta_detect) over the whole log; at
 N > 1 it ends when EVERY rank holds the joined, decoded match list of all ranks (siesta_exchange_*: the device-side
@@ -27,6 +28,7 @@ import numpy as np
 
 ROOT = os.path.dirname(os.path.abspath(__file__))
 sys.path.insert(0, ROOT)
+sys.dont_write_bytecode = True   # the bench writes nothing into the source tree, which may be read-only
 
 from sequencedetectionqueryexecutor_b200 import _abi as abi  # noqa: E402
 
@@ -92,6 +94,33 @@ WORKLOADS = {
 DEFAULT_WORKLOAD = "detection_gap6_100Mx50"
 CHUNK = 1_250_000      # traces per generator chunk: 100 M / 8 GPUs = 10 chunks, so every shard boundary is a chunk boundary
 SAMPLE_TRACES = 1_000_000   # the CPU arms (cpu_baseline, --impl reference) run the first SAMPLE_TRACES traces of the log
+DUMP_BYTES = 64_000_000     # --dump-outputs writes at most this many bytes in all
+DUMP_SEED = 0x51E57A00
+
+
+def dump_outputs(dm, device_index, out_dir):
+    """--dump-outputs: the columns a caller of the timed path receives (DeviceMatches.tensors(): matching trace ids, the
+    occurrence and event offsets, the event columns, the error and unsupported trace lists) as DIR/<column>.npy, and the
+    result sizes as DIR/sizes.npy.  An empty column (usually the error and unsupported lists) is not written: its length,
+    zero, is in sizes.npy.  float64 holds every value exactly (ids, offsets, positions and millisecond timestamps are
+    integers below 2**53).  A column longer than its share of DUMP_BYTES is written at a sorted sample of positions
+    drawn from (DUMP_SEED, its length), so two builds that compute the same result write the same files."""
+    import torch
+    cols = {k: t for k, t in dm.tensors(device_index).items() if t.numel()}
+    cap = (DUMP_BYTES - 4096 * (len(cols) + 1)) // (8 * max(len(cols), 1))   # 4096: room for each file's .npy header
+    os.makedirs(out_dir, exist_ok=True)
+    sizes = [dm.n_traces, dm.n_occurrences, dm.n_events, dm.n_matches_emitted, dm.n_ref_errors, dm.n_unsupported]
+    np.save(os.path.join(out_dir, "sizes.npy"), np.array(sizes, dtype=np.float64))
+    sampled = {}
+    for name, t in sorted(cols.items()):
+        n = t.numel()
+        if n > cap:
+            at = np.sort(np.random.default_rng([DUMP_SEED, n]).choice(n, cap, replace=False))
+            t = t[torch.from_numpy(at).to(t.device)]
+            sampled[name] = f"{cap} of {n}"
+        np.save(os.path.join(out_dir, f"{name}.npy"), t.to(torch.float64).cpu().numpy())
+    print(f"bench.py: wrote {len(cols) + 1} arrays to {out_dir}" + (f"; sampled: {sampled}" if sampled else ""),
+          file=sys.stderr, flush=True)
 
 
 def full_size_properties(log, nfa, flags, states, d_off, d_act, d_ts, device_index):
@@ -402,7 +431,12 @@ def main():
                          "(profiles/r02b_exchange_blocks.md)")
     ap.add_argument("--join", default="allgather", choices=["allgather", "none"],
                     help="N > 1: allgather = every rank ends the step with the decoded match list of all ranks")
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="write the result of the last timed step as DIR/<column>.npy (float64, at most 64 MB in all; "
+                         "a seeded sample of a longer column) to compare two builds output for output")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
     if args.warmup < 3:
         args.warmup = 3
     wl = dict(WORKLOADS[args.workload])
@@ -413,6 +447,10 @@ def main():
     rank = int(os.environ.get("RANK", "0"))
     local_rank = int(os.environ.get("LOCAL_RANK", "0"))
     world = int(os.environ.get("WORLD_SIZE", "1"))
+    if args.dump_outputs and args.impl == "reference":
+        ap.error("--dump-outputs writes the CUDA path's result (--impl b200)")
+    if args.dump_outputs and world > 1 and args.join != "allgather":
+        ap.error("--dump-outputs at N > 1 needs --join allgather: without it no rank holds the whole result")
 
     if args.impl == "reference":
         run_reference(args, wl, world, rank, emit)
@@ -486,7 +524,8 @@ def main():
 
     flush = torch.empty(512 << 20, dtype=torch.uint8, device=dev) if wl["bytes_per_event"] * E <= 2.6e8 else None
 
-    def step_resident():
+    def step_resident(keep=False):
+        """One request; keep=True returns its result (DeviceMatches) beside the sizes for the caller to close."""
         if flush is not None:
             flush.add_(1)  # inputs smaller than L2: evict them between steps
         if join is not None:
@@ -498,6 +537,8 @@ def main():
         else:
             dm = log.detect_device(nfa, flags=flags)
             out = (dm.n_traces, dm.n_occurrences, dm.n_events, dm.n_matches_emitted, dm.kernel_ms, dm.detect_ms, dm.n_traces, 0.0)
+        if keep:
+            return out, dm
         dm.close()
         return out
 
@@ -511,9 +552,13 @@ def main():
     k_ms, d_ms, x_ms, lat_ms = [], [], [], []
     barrier()
     t0 = time.perf_counter()
-    for _ in range(args.steps):
+    last = None     # --dump-outputs: the last timed step's result, written after the timed region
+    for i in range(args.steps):
         ts0 = time.perf_counter()
-        r = step_resident()
+        if args.dump_outputs and i == args.steps - 1:
+            r, last = step_resident(keep=True)
+        else:
+            r = step_resident()
         lat_ms.append((time.perf_counter() - ts0) * 1e3)
         k_ms.append(r[4])
         d_ms.append(r[5])
@@ -525,6 +570,10 @@ def main():
     launches = api.kernel_launches() - launches0
     clocks = sampler.stop()
     assert r[:4] == r0[:4], "result changed between steps"
+    if last is not None:
+        if rank == 0:     # at N > 1 every rank holds the same joined list of all ranks
+            dump_outputs(last, local_rank, args.dump_outputs)
+        last.close()
 
     t_step = torch.tensor([wall / args.steps], device=dev, dtype=torch.float64)
     if world > 1:
