@@ -200,6 +200,29 @@ int siesta_log_group(siesta_log* log, const int64_t* group_off, const int64_t* g
 /* Derived logs only: out[e] = index in the SOURCE log of event e (host array of siesta_log_n_events entries). */
 int siesta_log_source_events(siesta_log* log, int64_t* out);
 
+/* ------------------------------------------------------ growing a resident log */
+/* A new resident log = `log` with a batch of events appended, rebuilt on the device.  The batch is a CSR over the
+ * traces it touches: trace_idx[n_listed] strictly ascending LOCAL trace indices in [0, T + n_new_traces),
+ * batch_off[n_listed + 1] (batch_off[0] = 0, non-decreasing), act / ts_ms[batch_off[n_listed]].  The events of listed
+ * trace i go after the existing events of trace trace_idx[i], in the given order.  Indices >= T are new traces; new
+ * traces that are not listed are empty.  n_activities >= the log's (the dictionary only grows).  Activity ids outside
+ * [0, n_activities) are accepted as siesta_log_load accepts them; timestamps must stay sorted inside each trace (not
+ * checked, as in siesta_log_load).  The new log keeps the log's first_trace and owns its memory.
+ * `log` itself is NOT modified and stays valid: requests may keep running on it, and the caller frees it
+ * (siesta_log_free) when none does.  Peak device memory: the old log + the new log + the batch staging.
+ * SIESTA_E_INVALID (nothing changed, *out untouched): a null argument, trace indices not strictly ascending or out of
+ * range, n_new_traces < 0, malformed batch_off, n_activities below the log's, a derived log (siesta_log_filter_time /
+ * siesta_log_group) or a block-cyclic shard (siesta_log_set_blocks).  SIESTA_E_NOMEM: an allocation failed; the old
+ * log is intact.  *kernel_ms (may be NULL) = device time of the rebuild (CUDA events; excludes the host -> device copy
+ * of the batch).  The events are recorded on the context's stream, so work that other threads enqueue on the same
+ * context during the call is counted too; the time is the rebuild's alone only when nothing else runs on the context. */
+int siesta_log_append(siesta_log* log, const int64_t* trace_idx, const int64_t* batch_off, int64_t n_listed,
+                      const int32_t* act, const int64_t* ts_ms, int64_t n_new_traces, int32_t n_activities,
+                      siesta_log** out, double* kernel_ms);
+/* Host copy of traces [t0, t1) of a resident log: trace_off[t1 - t0 + 1] (offsets into the log's event columns, as
+ * stored), act / ts_ms[trace_off[t1-t0] - trace_off[0]] (both NULL: offsets only). */
+int siesta_log_read(siesta_log* log, int64_t t0, int64_t t1, int64_t* trace_off, int32_t* act, int64_t* ts_ms);
+
 /* -------------------------------------------------------------- detection */
 /* flags */
 #define SIESTA_F_RETURN_ALL 1u       /* Occurrences.clearOccurrences(true) (model/Occurrences.java:58-89) */
@@ -409,6 +432,13 @@ int siesta_multi_log_load(siesta_multi* m, const int64_t* trace_off, const int32
                           int64_t n_traces, int64_t n_events, int32_t n_activities, siesta_multi_log** out);
 void siesta_multi_log_free(siesta_multi_log* log);
 siesta_log* siesta_multi_log_shard(siesta_multi_log* log, int32_t shard); /* borrowed: any single-GPU call on one shard */
+/* siesta_log_append over a sharded log.  trace_idx are GLOBAL.  New traces go to the last shard (shards are not
+ * rebalanced).  Every shard is rebuilt on its device from its own host thread; a shard with no listed trace is
+ * copied, so the new multi log owns all of its shards.  The old multi log stays valid and unchanged; if one shard
+ * fails, the shards already built are freed and the error is returned. */
+int siesta_multi_log_append(siesta_multi_log* log, const int64_t* trace_idx, const int64_t* batch_off, int64_t n_listed,
+                            const int32_t* act, const int64_t* ts_ms, int64_t n_new_traces, int32_t n_activities,
+                            siesta_multi_log** out);
 /* = siesta_detect(whole log, nfa, NULL, 0, flags): SaseConnector.evaluate + clearOccurrences
  * (SaseConnection/SaseConnector.java:48-76), global trace indices, trace order. */
 int siesta_multi_detect(siesta_multi_log* log, const siesta_nfa* nfa, uint32_t flags, siesta_matches** out);

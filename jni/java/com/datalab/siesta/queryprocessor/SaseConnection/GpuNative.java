@@ -20,6 +20,9 @@ final class GpuNative {
     static native int[] patternCompile(int[] symbols, long[] constraints, boolean onlyAppearances);
     static native long logLoad(long multi, long[] traceOff, int[] act, long[] tsMs, int nActivities);
     static native void logFree(long log);
+    // a new resident log = `log` + a batch (events of traceIdx[i] = act / tsMs[batchOff[i] .. batchOff[i + 1]), global
+    // indices, >= the log's trace count for new traces); `log` stays valid until logFree
+    static native long logAppend(long log, long[] traceIdx, long[] batchOff, int[] act, long[] tsMs, long nNewTraces, int nActivities);
     static native long detect(long log, int[] nfa, int flags);
     static native long evaluateEvents(long multi, long[] traceOff, int[] act, long[] tsMs, int nActivities, int[] nfa, int flags);
     static native long[] matchesSizes(long matches);

@@ -29,6 +29,11 @@ static void throw_last(JNIEnv* env, const char* what) {
     if (rte) (*env)->ThrowNew(env, rte, msg);
 }
 
+static void throw_class(JNIEnv* env, const char* cls, const char* msg) {
+    jclass c = (*env)->FindClass(env, cls);
+    if (c) (*env)->ThrowNew(env, c, msg);
+}
+
 /* long init(int[] deviceIds): one process drives all GPUs (siesta_multi_init) */
 NATIVE(jlong, init)(JNIEnv* env, jclass cls, jintArray deviceIds) {
     (void)cls;
@@ -117,6 +122,51 @@ NATIVE(jlong, logLoad)(JNIEnv* env, jclass cls, jlong multi, jlongArray traceOff
         return 0;
     }
     return (jlong)(intptr_t)log;
+}
+
+/* long logAppend(long log, long[] traceIdx, long[] batchOff, int[] act, long[] tsMs, long nNewTraces, int nActivities):
+ * a new resident log with the batch appended (siesta_multi_log_append); the old handle stays valid until logFree.
+ * The arrays are copied out first (Get<Type>ArrayRegion), so none is pinned while the devices rebuild their shards. */
+NATIVE(jlong, logAppend)(JNIEnv* env, jclass cls, jlong log, jlongArray traceIdx, jlongArray batchOff, jintArray act, jlongArray tsMs,
+                         jlong nNewTraces, jint nActivities) {
+    (void)cls;
+    const jsize nl = (*env)->GetArrayLength(env, traceIdx), ne = (*env)->GetArrayLength(env, act);
+    int64_t* off = NULL;
+    if ((*env)->GetArrayLength(env, batchOff) == nl + 1) {
+        off = (int64_t*)malloc(sizeof(int64_t) * (size_t)(nl + 1));
+        if (!off) {
+            throw_class(env, "java/lang/OutOfMemoryError", "logAppend: host copy of the batch");
+            return 0;
+        }
+        (*env)->GetLongArrayRegion(env, batchOff, 0, nl + 1, (jlong*)off);
+    }
+    /* the library copies batchOff[nl] events: it must be exactly the arrays' length */
+    if (!off || (*env)->GetArrayLength(env, tsMs) != ne || off[nl] != (int64_t)ne) {
+        free(off);
+        throw_class(env, "java/lang/IllegalArgumentException",
+                    "logAppend: batchOff needs traceIdx.length + 1 entries ending at act.length, tsMs act.length entries");
+        return 0;
+    }
+    int64_t* idx = (int64_t*)malloc(sizeof(int64_t) * (size_t)(nl ? nl : 1));
+    int32_t* a = (int32_t*)malloc(sizeof(int32_t) * (size_t)(ne ? ne : 1));
+    int64_t* ts = (int64_t*)malloc(sizeof(int64_t) * (size_t)(ne ? ne : 1));
+    if (!idx || !a || !ts) {
+        free(off); free(idx); free(a); free(ts);
+        throw_class(env, "java/lang/OutOfMemoryError", "logAppend: host copy of the batch");
+        return 0;
+    }
+    (*env)->GetLongArrayRegion(env, traceIdx, 0, nl, (jlong*)idx);
+    (*env)->GetIntArrayRegion(env, act, 0, ne, (jint*)a);
+    (*env)->GetLongArrayRegion(env, tsMs, 0, ne, (jlong*)ts);
+    siesta_multi_log* out = NULL;
+    const int rc = siesta_multi_log_append((siesta_multi_log*)(intptr_t)log, idx, off, (int64_t)nl, a, ts, (int64_t)nNewTraces,
+                                           (int32_t)nActivities, &out);
+    free(off); free(idx); free(a); free(ts);
+    if (rc != SIESTA_OK) {
+        throw_last(env, "siesta_multi_log_append");
+        return 0;
+    }
+    return (jlong)(intptr_t)out;
 }
 
 NATIVE(void, logFree)(JNIEnv* env, jclass cls, jlong log) {

@@ -44,6 +44,8 @@ struct JNINativeInterface_ {
     void (*ReleaseLongArrayElements)(JNIEnv* env, jlongArray array, jlong* elems, jint mode);
     void (*SetIntArrayRegion)(JNIEnv* env, jintArray array, jsize start, jsize len, const jint* buf);
     void (*SetLongArrayRegion)(JNIEnv* env, jlongArray array, jsize start, jsize len, const jlong* buf);
+    void (*GetIntArrayRegion)(JNIEnv* env, jintArray array, jsize start, jsize len, jint* buf);
+    void (*GetLongArrayRegion)(JNIEnv* env, jlongArray array, jsize start, jsize len, jlong* buf);
     void* (*GetPrimitiveArrayCritical)(JNIEnv* env, jarray array, jboolean* isCopy);
     void (*ReleasePrimitiveArrayCritical)(JNIEnv* env, jarray array, void* carray, jint mode);
 };

@@ -25,6 +25,7 @@ EXPORTS = [
     "siesta_multi_init", "siesta_multi_shutdown", "siesta_multi_n_devices", "siesta_multi_log_load", "siesta_multi_log_free",
     "siesta_multi_log_shard", "siesta_multi_detect", "siesta_multi_declare_counts", "siesta_multi_why_not_match",
     "siesta_log_filter_time", "siesta_log_group", "siesta_log_source_events",
+    "siesta_log_append", "siesta_log_read", "siesta_multi_log_append",
 ]
 
 
@@ -123,6 +124,9 @@ def lib():
     L.siesta_log_filter_time.argtypes = [vp, i64, i32, i64, i32, P(vp)]
     L.siesta_log_group.argtypes = [vp, vp, vp, i32, vp, i32, P(vp), vp, P(i32)]
     L.siesta_log_source_events.argtypes = [vp, vp]
+    L.siesta_log_append.argtypes = [vp, vp, vp, i64, vp, vp, i64, i32, P(vp), P(C.c_double)]
+    L.siesta_log_read.argtypes = [vp, i64, i64, vp, vp, vp]
+    L.siesta_multi_log_append.argtypes = [vp, vp, vp, i64, vp, vp, i64, i32, P(vp)]
     L.siesta_device_free.argtypes = [vp, vp]
     L.siesta_device_free.restype = None
     _lib = L

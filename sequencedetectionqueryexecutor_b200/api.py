@@ -11,6 +11,19 @@ def _ptr(a):
     return C.c_void_p(a.ctypes.data) if a is not None else None
 
 
+def _batch(trace_idx, batch_off, act, ts_ms):
+    """An appended batch as the C-ABI takes it: (trace_idx int64, batch_off int64, act int32, ts_ms int64)."""
+    out = (np.ascontiguousarray(trace_idx, dtype=np.int64), np.ascontiguousarray(batch_off, dtype=np.int64),
+           np.ascontiguousarray(act, dtype=np.int32), np.ascontiguousarray(ts_ms, dtype=np.int64))
+    if len(out[1]) != len(out[0]) + 1:
+        raise ValueError("batch_off must have one entry more than trace_idx")
+    if len(out[2]) != len(out[3]):
+        raise ValueError("act and ts_ms must have the same length")
+    if out[1][-1] != len(out[2]):   # the library copies batch_off[-1] events: it must be exactly the arrays' length
+        raise ValueError(f"batch_off[-1] = {int(out[1][-1])} but act / ts_ms hold {len(out[2])} events")
+    return out
+
+
 class Context:
     """siesta_ctx: one per (process, device)."""
 
@@ -113,6 +126,28 @@ class EventLog:
         check(lib().siesta_log_group(self._h, _ptr(off), _ptr(flat) if len(flat) else None, len(groups), _ptr(ty), len(ty), C.byref(h),
                                      _ptr(gids), C.byref(k)))
         return EventLog._adopt(self.ctx, h, self.n_activities), gids[:k.value].copy()
+
+    def append(self, trace_idx, batch_off, act, ts_ms, n_new_traces=0, n_activities=None):
+        """siesta_log_append: a new resident EventLog = this log with the batch appended (events [batch_off[i],
+        batch_off[i + 1]) go after the events of trace trace_idx[i]; indices >= n_traces are new traces) ->
+        (EventLog, kernel_ms).  This log is not modified and stays usable; close it when no request needs it."""
+        ti, bo, a, ts = _batch(trace_idx, batch_off, act, ts_ms)
+        n_act = self.n_activities if n_activities is None else int(n_activities)
+        h, ms = C.c_void_p(), C.c_double(0.0)
+        check(lib().siesta_log_append(self._h, _ptr(ti), _ptr(bo), len(ti), _ptr(a), _ptr(ts), int(n_new_traces), n_act,
+                                      C.byref(h), C.byref(ms)))
+        return EventLog._adopt(self.ctx, h, n_act), ms.value
+
+    def read(self, t0=0, t1=None):
+        """siesta_log_read: host copy of traces [t0, t1) -> (trace_off as stored, act, ts_ms)."""
+        t1 = self.n_traces if t1 is None else int(t1)
+        off = np.zeros(max(t1 - int(t0), 0) + 1, dtype=np.int64)
+        check(lib().siesta_log_read(self._h, int(t0), t1, _ptr(off), None, None))
+        n = int(off[-1] - off[0])
+        act = np.zeros(max(n, 1), dtype=np.int32)
+        ts = np.zeros(max(n, 1), dtype=np.int64)
+        check(lib().siesta_log_read(self._h, int(t0), t1, _ptr(off), _ptr(act), _ptr(ts)))
+        return off, act[:n], ts[:n]
 
     def source_events(self):
         """Derived logs: index in the source log of every event."""
@@ -372,6 +407,18 @@ class MultiLog:
         self._h = C.c_void_p()
         check(lib().siesta_multi_log_load(multi._h, _ptr(trace_off), _ptr(act), _ptr(ts_ms), len(trace_off) - 1, len(act),
                                           self.n_activities, C.byref(self._h)))
+
+    def append(self, trace_idx, batch_off, act, ts_ms, n_new_traces=0, n_activities=None):
+        """siesta_multi_log_append: EventLog.append with GLOBAL trace indices; new traces go to the last shard ->
+        a new MultiLog (this one is not modified)."""
+        ti, bo, a, ts = _batch(trace_idx, batch_off, act, ts_ms)
+        n_act = self.n_activities if n_activities is None else int(n_activities)
+        h = C.c_void_p()
+        check(lib().siesta_multi_log_append(self._h, _ptr(ti), _ptr(bo), len(ti), _ptr(a), _ptr(ts), int(n_new_traces), n_act,
+                                            C.byref(h)))
+        new = MultiLog.__new__(MultiLog)
+        new.multi, new.n_activities, new._h = self.multi, n_act, h
+        return new
 
     def detect(self, nfa, flags=0):
         out = C.POINTER(_abi.Matches)()

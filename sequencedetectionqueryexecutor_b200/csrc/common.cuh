@@ -137,6 +137,9 @@ struct RebaseOffsets {
 int detect_device_impl(Log* log, const siesta_nfa* nfa, const int64_t* d_cand, int64_t n_cand, uint32_t flags, cudaStream_t stream,
                        RebaseOffsets base, siesta_dev_matches* out);
 int validate_act_range(Log* L, int64_t first_event, int64_t n_events, cudaStream_t stream);
+// Host checks of an appended batch against a log of T traces (siesta_log_append's rules; sets the error, append.cu)
+bool append_check_batch(const char* fn, int64_t T, const int64_t* trace_idx, const int64_t* batch_off, int64_t n_listed,
+                        const int32_t* act, const int64_t* ts_ms, int64_t n_new_traces);
 int assemble_matches(Ctx* c, std::vector<siesta_dev_matches>& parts, uint32_t flags, cudaStream_t stream, siesta_matches** out,
                      const std::vector<Ctx*>* part_ctx);
 int detect_device_finish_impl(DetectPending* q, siesta_dev_matches* out);

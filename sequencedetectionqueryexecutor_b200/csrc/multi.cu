@@ -1112,6 +1112,63 @@ extern "C" void siesta_multi_log_free(siesta_multi_log* lh) {
     delete ml;
 }
 
+// The batch is split by shard (new traces go to the last one) with its indices and offsets rebased, and every shard is
+// rebuilt by siesta_log_append on its device from its own host thread.  The old multi log is not touched.
+extern "C" int siesta_multi_log_append(siesta_multi_log* lh, const int64_t* trace_idx, const int64_t* batch_off, int64_t n_listed,
+                                       const int32_t* act, const int64_t* ts_ms, int64_t n_new_traces, int32_t n_activities,
+                                       siesta_multi_log** out) {
+    MultiLog* ml = reinterpret_cast<MultiLog*>(lh);
+    if (!ml || !out) {
+        set_error("siesta_multi_log_append: null argument");
+        return SIESTA_E_INVALID;
+    }
+    const int n = (int)ml->shard.size();
+    const int64_t total = ml->first[(size_t)n];
+    if (n_activities < ml->n_activities) {
+        set_error("siesta_multi_log_append: n_activities is smaller than the log's (the dictionary only grows)");
+        return SIESTA_E_INVALID;
+    }
+    if (!append_check_batch("siesta_multi_log_append", total, trace_idx, batch_off, n_listed, act, ts_ms, n_new_traces)) return SIESTA_E_INVALID;
+    // listed traces [cut[r], cut[r + 1]) belong to shard r
+    std::vector<int64_t> cut((size_t)n + 1, n_listed);
+    cut[0] = 0;
+    for (int r = 1; r < n; ++r) cut[(size_t)r] = (int64_t)(std::lower_bound(trace_idx, trace_idx + n_listed, ml->first[(size_t)r]) - trace_idx);
+    std::vector<Log*> built((size_t)n, nullptr);
+    std::vector<int> rcs((size_t)n, SIESTA_OK);
+    std::vector<std::string> errs((size_t)n);
+    {
+        std::vector<std::thread> th;
+        for (int r = 0; r < n; ++r)
+            th.emplace_back([&, r] {
+                const int64_t l0 = cut[(size_t)r], l1 = cut[(size_t)r + 1], b0 = batch_off[l0];
+                std::vector<int64_t> idx((size_t)(l1 - l0)), off((size_t)(l1 - l0 + 1));
+                for (int64_t i = l0; i < l1; ++i) idx[(size_t)(i - l0)] = trace_idx[i] - ml->first[(size_t)r];
+                for (int64_t i = l0; i <= l1; ++i) off[(size_t)(i - l0)] = batch_off[i] - b0;
+                siesta_log* lg = nullptr;
+                rcs[(size_t)r] = siesta_log_append(reinterpret_cast<siesta_log*>(ml->shard[(size_t)r]), idx.data(), off.data(), l1 - l0,
+                                                   act ? act + b0 : nullptr, ts_ms ? ts_ms + b0 : nullptr, r == n - 1 ? n_new_traces : 0,
+                                                   n_activities, &lg, nullptr);
+                if (rcs[(size_t)r] == SIESTA_OK) built[(size_t)r] = reinterpret_cast<Log*>(lg);
+                else errs[(size_t)r] = siesta_last_error();
+            });
+        for (std::thread& t : th) t.join();
+    }
+    for (int r = 0; r < n; ++r)
+        if (rcs[(size_t)r] != SIESTA_OK) {
+            for (Log* l : built) siesta_log_free(reinterpret_cast<siesta_log*>(l));
+            set_error(errs[(size_t)r]);
+            return rcs[(size_t)r];
+        }
+    MultiLog* nl = new MultiLog();
+    nl->m = ml->m;
+    nl->shard = built;
+    nl->first = ml->first;
+    nl->first[(size_t)n] = total + n_new_traces;
+    nl->n_activities = n_activities;
+    *out = reinterpret_cast<siesta_multi_log*>(nl);
+    return SIESTA_OK;
+}
+
 extern "C" siesta_log* siesta_multi_log_shard(siesta_multi_log* lh, int32_t r) {
     MultiLog* ml = reinterpret_cast<MultiLog*>(lh);
     return (ml && r >= 0 && r < (int)ml->shard.size()) ? reinterpret_cast<siesta_log*>(ml->shard[(size_t)r]) : nullptr;

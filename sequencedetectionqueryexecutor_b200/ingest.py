@@ -88,6 +88,94 @@ def read_seq_table(src, activities: Optional[ActivityDictionary] = None, tz_offs
     return SeqLog(trace_off, np.ascontiguousarray(act[order]), np.ascontiguousarray(ts[order]), trace_ids, acts)
 
 
+@dataclass
+class SeqDelta:
+    """A batch of events to append to a resident log (EventLog.append / MultiLog.append take its fields): the events of
+    listed trace i are act / ts_ms[batch_off[i]:batch_off[i + 1]] and go after the existing events of trace
+    trace_idx[i] (ascending); indices >= the log's trace count are new traces."""
+    trace_idx: np.ndarray          # int64 [k] ascending dense trace indices
+    batch_off: np.ndarray          # int64 [k + 1]
+    act: np.ndarray                # int32 [batch_off[k]]
+    ts_ms: np.ndarray              # int64 [batch_off[k]]
+    n_new_traces: int
+    n_activities: int              # size of the (grown) activity dictionary
+
+
+def read_seq_delta(src, trace_ids: List[str], activities: ActivityDictionary, trace_lens=None, tz_offset_ms=0) -> SeqDelta:
+    """A seq.parquet batch the preprocess wrote after the log became resident -> SeqDelta.  Known trace ids map to their
+    dense index; unknown ones are numbered T, T + 1, ... in order of first appearance and appended to `trace_ids`.
+    Names go through the same case-folding `activities`, which grows.  Events are ordered by `position`, ties by table
+    order (as read_seq_table).  With `trace_lens` (current event count of every known trace), a row whose position lies
+    below its trace's length raises ValueError: such a batch rewrites existing events, which an append cannot."""
+    tb = _table(src, ["trace_id", "event_type", "timestamp", "position"])
+    n, T = tb.num_rows, len(trace_ids)
+    if n == 0:
+        return SeqDelta(np.zeros(0, dtype=np.int64), np.zeros(1, dtype=np.int64), np.zeros(0, dtype=np.int32),
+                        np.zeros(0, dtype=np.int64), 0, len(activities))
+    index_of = {t: i for i, t in enumerate(trace_ids)}
+    tid_dict = tb["trace_id"].combine_chunks().dictionary_encode()
+    n_new = 0
+    dense = []
+    for x in tid_dict.dictionary.to_pylist():                         # dictionary order = first appearance
+        x = str(x)
+        if x not in index_of:
+            index_of[x] = T + n_new
+            trace_ids.append(x)
+            n_new += 1
+        dense.append(index_of[x])
+    tr = np.asarray(dense, dtype=np.int64)[np.asarray(tid_dict.indices, dtype=np.int64)]
+    ev_dict = tb["event_type"].combine_chunks().dictionary_encode()
+    name_to_id = np.array([activities.add(str(x)) for x in ev_dict.dictionary.to_pylist()], dtype=np.int32)
+    act = name_to_id[np.asarray(ev_dict.indices, dtype=np.int64)]
+    ts = timestamps_to_ms(tb["timestamp"], tz_offset_ms)
+    pos = np.asarray(tb["position"].combine_chunks().to_numpy(zero_copy_only=False), dtype=np.int64)
+    if trace_lens is not None and T:
+        lens = np.asarray(trace_lens, dtype=np.int64)
+        known = tr < T
+        bad = np.zeros(n, dtype=bool)
+        bad[known] = pos[known] < lens[tr[known]]
+        if bad.any():
+            r = int(np.flatnonzero(bad)[0])
+            raise ValueError(f"batch row {r} rewrites position {int(pos[r])} of trace {trace_ids[int(tr[r])]!r}, "
+                             f"which already holds {int(lens[tr[r]])} events: not an append")
+    order = np.lexsort((np.arange(n), pos, tr))                      # by trace, then position, then table order
+    trace_idx, counts = np.unique(tr, return_counts=True)
+    batch_off = np.zeros(len(trace_idx) + 1, dtype=np.int64)
+    np.cumsum(counts, out=batch_off[1:])
+    return SeqDelta(trace_idx.astype(np.int64), batch_off, np.ascontiguousarray(act[order]), np.ascontiguousarray(ts[order]),
+                    n_new, len(activities))
+
+
+def merge_delta(trace_off, act, ts_ms, delta: SeqDelta):
+    """The append restated on the host: (trace_off, act, ts_ms) of the log with `delta` appended - what
+    siesta_log_append builds on the device, and the host copy a caller that keeps one maintains."""
+    trace_off = np.asarray(trace_off, dtype=np.int64)
+    T = len(trace_off) - 1
+    T2 = T + int(delta.n_new_traces)
+    old_len = np.zeros(T2, dtype=np.int64)
+    old_len[:T] = np.diff(trace_off)
+    add = np.zeros(T2, dtype=np.int64)
+    add[delta.trace_idx] = np.diff(delta.batch_off)
+    new_off = np.zeros(T2 + 1, dtype=np.int64)
+    np.cumsum(old_len + add, out=new_off[1:])
+    E2 = int(new_off[-1])
+    # destination of every old event (shifted by the batch events of earlier traces) and of every batch event
+    before = np.zeros(T2 + 1, dtype=np.int64)
+    np.cumsum(add, out=before[1:])
+    old_trace = np.repeat(np.arange(T), old_len[:T])
+    old_dst = np.arange(int(trace_off[-1]), dtype=np.int64) + before[old_trace]
+    b_trace = np.repeat(delta.trace_idx, np.diff(delta.batch_off))
+    b_rank = np.arange(int(delta.batch_off[-1]), dtype=np.int64) - np.repeat(delta.batch_off[:-1], np.diff(delta.batch_off))
+    b_dst = new_off[b_trace] + old_len[b_trace] + b_rank
+    out_act = np.zeros(E2, dtype=np.int32)
+    out_ts = np.zeros(E2, dtype=np.int64)
+    out_act[old_dst] = act
+    out_ts[old_dst] = ts_ms
+    out_act[b_dst] = delta.act
+    out_ts[b_dst] = delta.ts_ms
+    return new_off, out_act, out_ts
+
+
 def read_index_table(src, log: SeqLog, pairs: Optional[Sequence[Tuple[str, str]]] = None):
     """index.parquet -> (pairs [(activity id A, activity id B)], posting lists [ascending int64 dense trace indices]),
     ready for EventLog.load_index.  `pairs` (names) restricts the read to the requested pairs, as getAllEventPairs'
