@@ -146,7 +146,7 @@ typedef struct siesta_log siesta_log;
 
 /* One ctx per (process, device).  Multi-GPU = one ctx per GPU; the traces
  * shard by contiguous trace range and the exchange step (match-list
- * all-gather, count all-reduce) runs over NCCL one level up. */
+ * all-gather, count all-reduce) is siesta_exchange_* (below). */
 int siesta_init(int32_t device_id, siesta_ctx** out);
 void siesta_shutdown(siesta_ctx* ctx);
 
@@ -303,7 +303,7 @@ int siesta_evaluate_events_act8(siesta_ctx* ctx, const int64_t* trace_off, const
                                 int32_t n_activities, const siesta_nfa* nfa, uint32_t flags,
                                 siesta_matches** out);
 
-/* Device-level variant used by the torch/NCCL layer: results stay in HBM.
+/* Device-level variant for callers that consume the result on the device: results stay in HBM.
  * All pointers are device pointers owned by the library until
  * siesta_dev_matches_free; `stream` is a cudaStream_t (NULL = the ctx stream). */
 typedef struct siesta_dev_matches {
@@ -319,8 +319,7 @@ typedef struct siesta_dev_matches {
     double kernel_ms;
     double detect_ms;
     /* all eight arrays above live in ONE device allocation [d_block, d_block + block_bytes), each at a 256-byte
-     * aligned offset, in the order trace_idx, occ_off, ev_off, ev_pos, err_trace_idx, ev_rank, ev_act, ev_ts_ms:
-     * the multi-GPU exchange ships the block with a single all-gather */
+     * aligned offset, in the order trace_idx, occ_off, ev_off, ev_pos, err_trace_idx, ev_rank, ev_act, ev_ts_ms */
     void* d_block;
     int64_t block_bytes;
     void* impl;
@@ -341,16 +340,6 @@ int siesta_detect_device_begin(siesta_log* log, const siesta_nfa* nfa, const int
                                uint32_t flags, void* stream, siesta_detect_pending** out);
 int siesta_detect_device_finish(siesta_detect_pending* pending, siesta_dev_matches* out);
 void siesta_dev_matches_free(siesta_dev_matches* m);
-
-/* Compact wire format of a device result for the multi-GPU exchange (13 B per trace + 1 B per occurrence + 9 B per
- * event instead of 24 + 8 + 20; layout: csrc/explore.cu, decoder: distributed.unpack_block).  d_out is device memory of
- * at least siesta_packed_block_bytes(...) bytes; `stream` a cudaStream_t (NULL = ctx stream).  trace_base is
- * subtracted from trace_idx (the shard's first trace).  Returns SIESTA_E_UNSUPPORTED when a value does not fit
- * (activity id >= 65 536, a timestamp delta outside int32 ...): ship the plain block (d_block) then. */
-int64_t siesta_packed_block_bytes(int64_t n_traces, int64_t n_occurrences, int64_t n_events, int64_t n_ref_errors,
-                                  int32_t has_event_columns);
-int siesta_dev_matches_pack(siesta_log* log, const siesta_dev_matches* m, uint32_t flags, int64_t trace_base,
-                            void* d_out, int64_t out_bytes, void* stream);
 
 /* ------------------------------------------------------- multi-GPU exchange */
 /* Traces are independent, so a log shards by contiguous trace range, one shard per GPU (siesta_log_set_first_trace),

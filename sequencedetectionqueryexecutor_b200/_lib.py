@@ -19,7 +19,6 @@ EXPORTS = [
     "siesta_intersect", "siesta_intersect_device", "siesta_device_free", "siesta_pattern_extract_pairs",
     "siesta_candidates", "siesta_candidates_device", "siesta_pair_stats", "siesta_pair_stats_device",
     "siesta_explore_accurate", "siesta_why_not_match", "siesta_almost_matches_free", "siesta_log_set_first_trace", "siesta_log_set_blocks",
-    "siesta_packed_block_bytes", "siesta_dev_matches_pack",
     "siesta_exchange_create", "siesta_exchange_export", "siesta_exchange_import", "siesta_exchange_connect_local",
     "siesta_exchange_free", "siesta_exchange_required_bytes", "siesta_detect_allgather", "siesta_exchange_allreduce_i64",
     "siesta_multi_init", "siesta_multi_shutdown", "siesta_multi_n_devices", "siesta_multi_log_load", "siesta_multi_log_free",
@@ -52,9 +51,6 @@ def lib():
     L.siesta_shutdown.restype = None
     L.siesta_log_load.argtypes = [vp, vp, vp, vp, i64, i64, i32, P(vp)]
     L.siesta_log_wrap_device.argtypes = [vp, vp, vp, vp, i64, i64, i32, i32, P(vp)]
-    L.siesta_packed_block_bytes.argtypes = [i64, i64, i64, i64, i32]
-    L.siesta_packed_block_bytes.restype = i64
-    L.siesta_dev_matches_pack.argtypes = [vp, P(_abi.DevMatches), u32, i64, vp, i64, vp]
     L.siesta_log_set_first_trace.argtypes = [vp, i64]
     L.siesta_log_set_first_trace.restype = None
     L.siesta_log_set_blocks.argtypes = [vp, i32, P(i64), P(i64)]

@@ -486,37 +486,6 @@ class DeviceMatches:
             lib().siesta_dev_matches_free(C.byref(self.dm))
             self.dm = None
 
-    def block(self, device_index=0):
-        """The whole result as one uint8 CUDA tensor (zero-copy view of the library's allocation; valid until close())
-        plus its header (n_traces, n_occurrences, n_events, n_ref_errors, has_event_columns); see distributed.py."""
-        import torch
-
-        class _View:
-            def __init__(self, ptr, n):
-                self.__cuda_array_interface__ = {"shape": (n,), "typestr": "|u1", "data": (ptr, False), "version": 2}
-
-        d = self.dm
-        t = (torch.as_tensor(_View(d.d_block, d.block_bytes), device=f"cuda:{device_index}") if d.block_bytes
-             else torch.zeros(0, dtype=torch.uint8, device=f"cuda:{device_index}"))
-        return t, (d.n_traces, d.n_occurrences, d.n_events, d.n_ref_errors, 1 if d.d_ev_rank else 0)
-
-    def packed_block(self, log, flags=0, trace_base=0, device_index=0):
-        """siesta_dev_matches_pack: the result in the compact wire format of the multi-GPU exchange -> (uint8 CUDA
-        tensor, header) for distributed.exchange_blocks, or None when a value does not fit (ship block() then)."""
-        import torch
-        d = self.dm
-        all_cols = 1 if d.d_ev_rank else 0
-        n = lib().siesta_packed_block_bytes(d.n_traces, d.n_occurrences, d.n_events, d.n_ref_errors, all_cols)
-        out = torch.empty(max(n, 1), dtype=torch.uint8, device=f"cuda:{device_index}")
-        stream = torch.cuda.current_stream(out.device).cuda_stream
-        rc = lib().siesta_dev_matches_pack(log._h, C.byref(d), flags, int(trace_base), C.c_void_p(out.data_ptr()), n,
-                                           C.c_void_p(stream))
-        if rc == _abi.E_UNSUPPORTED:
-            return None
-        check(rc)
-        return out[:n], (d.n_traces, d.n_occurrences, d.n_events, d.n_ref_errors, all_cols, 1, int(trace_base),
-                         0 if flags & _abi.F_EVT_POS else 1)
-
     def tensors(self, device_index=0):
         """Zero-copy torch views of the device result (valid until close()); keys as in MatchResult."""
         import torch

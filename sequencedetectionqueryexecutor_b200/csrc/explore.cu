@@ -334,150 +334,3 @@ extern "C" int siesta_explore_accurate(siesta_log* log, const int32_t* pattern_a
     if (kernel_ms) *kernel_ms = ms;
     return rc;
 }
-
-// ------------------------------------------------------------------------------------------- compact wire format
-// The multi-GPU exchange ships every rank's match list to every other rank: on configs[1] that is 104 MB per rank for
-// 1.2 GB scanned, and at eight GPUs the all-gather, not the scan, bounds the request.  siesta_dev_matches_pack rewrites a
-// result into narrow columns (sections at 256-byte aligned offsets, in this order):
-//   trace_local i32[n_tr]   trace_idx - trace_base            occ_cnt u8[n_tr]     occurrences of the trace (<= 64)
-//   ev_cnt      u8[n_occ]   events of the occurrence (<= 64)  ev_pos  u16[n_ev]    in-trace index (< 65 536)
-//   err         i64[n_err]                                    ev_rank u8[n_ev]     ev_act u16[n_ev]
-//   ts_base     i64[n_tr]   ev_ts_ms of the trace's first reported event
-//   ts_delta    i32[n_ev]   (ev_ts_ms - ts_base) / 1000 (EventTs route: exact, both are rel_s * 1000 + t0) or the raw
-//                           difference in ms (EventPos route)
-// = 13 B per trace + 1 B per occurrence + 9 B per event instead of 24 + 8 + 20.  Anything that does not fit (activity id
-// >= 65 536, a delta outside int32, a shard of >= 2^31 traces) makes the call fail with SIESTA_E_UNSUPPORTED and the
-// caller ships the plain block.  distributed.py decodes (`unpack_block`).
-namespace siesta {
-
-struct PackParams {
-    const int64_t* trace_idx;
-    const int64_t* occ_off;
-    const int64_t* ev_off;
-    const int32_t* ev_pos;
-    const int32_t* ev_rank;
-    const int32_t* ev_act;
-    const int64_t* ev_ts;
-    int64_t n_tr, n_occ, n_ev, trace_base;
-    int32_t seconds;  // ts_delta in seconds (EventTs route) or milliseconds
-    int32_t* o_trace;
-    uint8_t* o_occ_cnt;
-    uint8_t* o_ev_cnt;
-    uint16_t* o_pos;
-    uint8_t* o_rank;
-    uint16_t* o_act;
-    int64_t* o_base;
-    int32_t* o_delta;
-    int* bad;
-};
-
-__global__ void __launch_bounds__(256) pack_traces_kernel(const __grid_constant__ PackParams P) {
-    for (int64_t t = (int64_t)blockIdx.x * blockDim.x + threadIdx.x; t < P.n_tr; t += (int64_t)gridDim.x * blockDim.x) {
-        const int64_t local = P.trace_idx[t] - P.trace_base;
-        const int64_t o0 = P.occ_off[t], o1 = P.occ_off[t + 1];
-        if (local < 0 || local > 0x7fffffffll || o1 - o0 > 255) *P.bad = 1;
-        P.o_trace[t] = (int32_t)local;
-        P.o_occ_cnt[t] = (uint8_t)(o1 - o0);
-        const int64_t e0 = P.ev_off[o0];
-        const long long base = P.ev_ts ? P.ev_ts[e0] : 0;
-        if (P.o_base) P.o_base[t] = base;
-        for (int64_t o = o0; o < o1; ++o) {
-            const int64_t a = P.ev_off[o], b = P.ev_off[o + 1];
-            if (b - a > 255) *P.bad = 1;
-            P.o_ev_cnt[o] = (uint8_t)(b - a);
-            if (P.ev_ts)
-                for (int64_t e = a; e < b; ++e) {
-                    long long d = P.ev_ts[e] - base;
-                    if (P.seconds) {
-                        if (d % 1000 != 0) *P.bad = 1;
-                        d /= 1000;
-                    }
-                    if (d < -0x7fffffffll - 1 || d > 0x7fffffffll) *P.bad = 1;
-                    P.o_delta[e] = (int32_t)d;
-                }
-        }
-    }
-}
-
-__global__ void __launch_bounds__(256) pack_events_kernel(const __grid_constant__ PackParams P) {
-    for (int64_t e = (int64_t)blockIdx.x * blockDim.x + threadIdx.x; e < P.n_ev; e += (int64_t)gridDim.x * blockDim.x) {
-        const int32_t pos = P.ev_pos[e];
-        if ((unsigned)pos > 0xffffu) *P.bad = 1;
-        P.o_pos[e] = (uint16_t)pos;
-        if (P.ev_rank) {
-            const int32_t r = P.ev_rank[e], a = P.ev_act[e];
-            if ((unsigned)r > 0xffu || (unsigned)a > 0xffffu) *P.bad = 1;
-            P.o_rank[e] = (uint8_t)r;
-            P.o_act[e] = (uint16_t)a;
-        }
-    }
-}
-
-}  // namespace siesta
-
-static size_t al256(size_t x) { return (x + 255) & ~(size_t)255; }
-
-extern "C" int64_t siesta_packed_block_bytes(int64_t n_tr, int64_t n_occ, int64_t n_ev, int64_t n_err, int32_t all_cols) {
-    size_t b = al256((size_t)n_tr * 4) + al256((size_t)n_tr) + al256((size_t)n_occ) + al256((size_t)n_ev * 2) + al256((size_t)n_err * 8);
-    if (all_cols) b += al256((size_t)n_ev) + al256((size_t)n_ev * 2) + al256((size_t)n_tr * 8) + al256((size_t)n_ev * 4);
-    return (int64_t)b;
-}
-
-extern "C" int siesta_dev_matches_pack(siesta_log* log, const siesta_dev_matches* m, uint32_t flags, int64_t trace_base,
-                                       void* d_out, int64_t out_bytes, void* stream_) {
-    Log* L = reinterpret_cast<Log*>(log);
-    if (!L || !m || !d_out) {
-        set_error("siesta_dev_matches_pack: null argument");
-        return SIESTA_E_INVALID;
-    }
-    const int all_cols = m->d_ev_rank ? 1 : 0;
-    if (out_bytes < siesta_packed_block_bytes(m->n_traces, m->n_occurrences, m->n_events, m->n_ref_errors, all_cols)) {
-        set_error("siesta_dev_matches_pack: output buffer too small");
-        return SIESTA_E_INVALID;
-    }
-    SIESTA_CUDA_OK(cudaSetDevice(L->ctx->device));
-    cudaStream_t stream = stream_ ? reinterpret_cast<cudaStream_t>(stream_) : L->ctx->stream;
-    char* o = reinterpret_cast<char*>(d_out);
-    PackParams P;
-    std::memset(&P, 0, sizeof(P));
-    P.trace_idx = m->d_trace_idx; P.occ_off = m->d_occ_off; P.ev_off = m->d_ev_off; P.ev_pos = m->d_ev_pos;
-    P.ev_rank = m->d_ev_rank; P.ev_act = m->d_ev_act; P.ev_ts = m->d_ev_ts_ms;
-    P.n_tr = m->n_traces; P.n_occ = m->n_occurrences; P.n_ev = m->n_events; P.trace_base = trace_base;
-    P.seconds = (flags & SIESTA_F_EVT_POS) ? 0 : 1;
-    P.o_trace = reinterpret_cast<int32_t*>(o); o += al256((size_t)P.n_tr * 4);
-    P.o_occ_cnt = reinterpret_cast<uint8_t*>(o); o += al256((size_t)P.n_tr);
-    P.o_ev_cnt = reinterpret_cast<uint8_t*>(o); o += al256((size_t)P.n_occ);
-    P.o_pos = reinterpret_cast<uint16_t*>(o); o += al256((size_t)P.n_ev * 2);
-    char* o_err = o; o += al256((size_t)m->n_ref_errors * 8);
-    if (all_cols) {
-        P.o_rank = reinterpret_cast<uint8_t*>(o); o += al256((size_t)P.n_ev);
-        P.o_act = reinterpret_cast<uint16_t*>(o); o += al256((size_t)P.n_ev * 2);
-        P.o_base = reinterpret_cast<int64_t*>(o); o += al256((size_t)P.n_tr * 8);
-        P.o_delta = reinterpret_cast<int32_t*>(o);
-    }
-    int* d_bad = nullptr;
-    SIESTA_CUDA_OK(cudaMallocAsync((void**)&d_bad, sizeof(int), stream));
-    SIESTA_CUDA_OK(cudaMemsetAsync(d_bad, 0, sizeof(int), stream));
-    P.bad = d_bad;
-    if (m->n_ref_errors)
-        SIESTA_CUDA_OK(cudaMemcpyAsync(o_err, m->d_err_trace_idx, (size_t)m->n_ref_errors * 8, cudaMemcpyDeviceToDevice, stream));
-    const int cap = L->ctx->sm_count * 8;
-    if (P.n_tr > 0) {
-        pack_traces_kernel<<<(int)std::min<int64_t>((P.n_tr + 255) / 256, cap), 256, 0, stream>>>(P);
-        SIESTA_LAUNCHED();
-    }
-    if (P.n_ev > 0) {
-        pack_events_kernel<<<(int)std::min<int64_t>((P.n_ev + 255) / 256, cap), 256, 0, stream>>>(P);
-        SIESTA_LAUNCHED();
-    }
-    SIESTA_CUDA_OK(cudaGetLastError());
-    int bad = 0;
-    SIESTA_CUDA_OK(cudaMemcpyAsync(&bad, d_bad, sizeof(int), cudaMemcpyDeviceToHost, stream));
-    SIESTA_CUDA_OK(cudaStreamSynchronize(stream));
-    cudaFreeAsync(d_bad, stream);
-    if (bad) {
-        set_error("siesta_dev_matches_pack: a value does not fit the compact wire format; ship the plain block");
-        return SIESTA_E_UNSUPPORTED;
-    }
-    return SIESTA_OK;
-}

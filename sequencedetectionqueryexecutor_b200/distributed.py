@@ -1,14 +1,13 @@
 """Multi-GPU plumbing: one process per GPU, traces sharded by contiguous trace range (SURVEY.md §8e).
 
-The scan itself has no exchange step: every rank verifies / counts its own shard.  Two collectives join the
-results over NCCL (NVLink 5 / NVSwitch): an all-gather of the per-rank match lists (/detection) and a sum
-all-reduce of the packed int64 count array (/declare, /stats).  Both are latency-bound (outputs are a few
-percent of the scan), so they are issued once per request on padded buffers.
-
-Works on CPU tensors with the gloo backend too (tests/test_distributed_cpu.py).
+The scan itself has no exchange step: every rank verifies / counts its own shard.  The results are joined afterwards:
+- /detection: MatchExchange sets up the library's exchange (siesta_exchange_*, csrc/multi.cu) over torch.distributed;
+  every request then all-gathers the per-rank match lists on the devices, over NVLink peer memory.
+- /declare, /stats: a sum all-reduce of the packed int64 count array, on the devices (MatchExchange.allreduce_counts) or
+  through torch.distributed (allreduce_counts, allreduce_pair_stats; these also work on CPU tensors with the gloo
+  backend, tests/test_distributed_cpu.py).
 """
 import numpy as np
-import os
 
 import torch
 import torch.distributed as dist
@@ -33,290 +32,6 @@ def local_shard(trace_off, act, ts_ms, rank, world):
     lo, hi = int(b[rank]), int(b[rank + 1])
     e0, e1 = int(trace_off[lo]), int(trace_off[hi])
     return (np.asarray(trace_off[lo:hi + 1], dtype=np.int64) - e0, np.asarray(act[e0:e1]), np.asarray(ts_ms[e0:e1]), lo)
-
-
-def _gather_var(t, group=None):
-    """all-gather of 1-D tensors of different lengths: sizes first, then one padded all-gather."""
-    world = dist.get_world_size(group)
-    n = torch.tensor([t.numel()], dtype=torch.int64, device=t.device)
-    sizes = [torch.zeros_like(n) for _ in range(world)]
-    dist.all_gather(sizes, n, group=group)
-    sizes = [int(s.item()) for s in sizes]
-    m = max(max(sizes), 1)
-    pad = torch.zeros(m, dtype=t.dtype, device=t.device)
-    pad[:t.numel()] = t
-    outs = [torch.empty_like(pad) for _ in range(world)]
-    dist.all_gather(outs, pad, group=group)
-    return [o[:s] for o, s in zip(outs, sizes)]
-
-
-def allgather_matches(local, first_trace, group=None):
-    """Join per-rank match lists (dict of 1-D tensors: trace_idx, occ_off, ev_off, ev_pos[, ev_rank, ev_act, ev_ts_ms],
-    err_trace_idx; indices local to the shard) into the global CSR, identical on every rank.  Ranks own ascending,
-    disjoint trace ranges, so concatenating in rank order keeps trace_idx ascending."""
-    cols = [k for k in ("ev_pos", "ev_rank", "ev_act", "ev_ts_ms") if local.get(k) is not None]
-    tr = _gather_var(local["trace_idx"] + first_trace, group)
-    err = _gather_var(local["err_trace_idx"] + first_trace, group)
-    occ_cnt = _gather_var(local["occ_off"][1:] - local["occ_off"][:-1], group)
-    ev_cnt = _gather_var(local["ev_off"][1:] - local["ev_off"][:-1], group)
-    out = {"trace_idx": torch.cat(tr), "err_trace_idx": torch.cat(err)}
-    for name, parts in (("occ_off", occ_cnt), ("ev_off", ev_cnt)):
-        c = torch.cat(parts)
-        off = torch.zeros(c.numel() + 1, dtype=torch.int64, device=c.device)
-        torch.cumsum(c, 0, out=off[1:])
-        out[name] = off
-    for k in cols:
-        out[k] = torch.cat(_gather_var(local[k], group))
-    return out
-
-
-# ---------------------------------------------------------------------------------------------- block exchange
-# siesta_dev_matches keeps a result in ONE allocation (include/siesta_gpu.h): eight arrays at 256-byte aligned
-# offsets.  The /detection exchange ships that block as it is: a header all-gather (5 int64 per rank), one copy of
-# the own block into the receive buffer, one padded all-gather of bytes.  The joined match list is the sequence of
-# per-rank parts (each a self-contained CSR with GLOBAL trace indices, see siesta_log_set_first_trace); ranks own
-# ascending disjoint trace ranges, so the parts in rank order are the trace-ordered result.  Nothing is re-packed,
-# and the all-gather may still be in flight when the next request's kernels start (JoinedMatches.wait()).
-
-def _align256(n):
-    return (n + 255) & ~255
-
-
-def block_layout(n_tr, n_occ, n_ev, n_err, all_cols):
-    """Byte offsets of the arrays inside a result block (mirror of detect_device_impl's carve order)."""
-    off, o = {}, 0
-    for name, nbytes in (("trace_idx", n_tr * 8), ("occ_off", (n_tr + 1) * 8), ("ev_off", (n_occ + 1) * 8), ("ev_pos", n_ev * 4),
-                         ("err_trace_idx", n_err * 8)):
-        off[name] = (o, nbytes)
-        o += _align256(nbytes)
-    if all_cols:
-        for name, nbytes in (("ev_rank", n_ev * 4), ("ev_act", n_ev * 4), ("ev_ts_ms", n_ev * 8)):
-            off[name] = (o, nbytes)
-            o += _align256(nbytes)
-    return off, o
-
-
-_DT = {"trace_idx": torch.int64, "occ_off": torch.int64, "ev_off": torch.int64, "ev_pos": torch.int32,
-       "err_trace_idx": torch.int64, "ev_rank": torch.int32, "ev_act": torch.int32, "ev_ts_ms": torch.int64}
-
-
-def packed_layout(n_tr, n_occ, n_ev, n_err, all_cols):
-    """Byte offsets inside a compact block (mirror of siesta_dev_matches_pack, csrc/explore.cu)."""
-    off, o = {}, 0
-    secs = [("trace_local", n_tr * 4), ("occ_cnt", n_tr), ("ev_cnt", n_occ), ("ev_pos", n_ev * 2), ("err_trace_idx", n_err * 8)]
-    if all_cols:
-        secs += [("ev_rank", n_ev), ("ev_act", n_ev * 2), ("ts_base", n_tr * 8), ("ts_delta", n_ev * 4)]
-    for name, nbytes in secs:
-        off[name] = (o, nbytes)
-        o += _align256(nbytes)
-    return off, o
-
-
-_PDT = {"trace_local": torch.int32, "occ_cnt": torch.uint8, "ev_cnt": torch.uint8, "ev_pos": torch.int16,
-        "err_trace_idx": torch.int64, "ev_rank": torch.uint8, "ev_act": torch.int16, "ts_base": torch.int64,
-        "ts_delta": torch.int32}
-
-
-def unpack_block(row, header):
-    """Compact block -> the standard columns (dict of tensors, global trace indices)."""
-    n_tr, n_occ, n_ev, n_err, all_cols, fmt, trace_base, seconds = header[:8]
-    lay, _ = packed_layout(n_tr, n_occ, n_ev, n_err, all_cols)
-    v = {k: row[o:o + nb].view(_PDT[k]) for k, (o, nb) in lay.items()}
-    dev = row.device
-
-    def offsets(cnt, n):
-        off = torch.zeros(n + 1, dtype=torch.int64, device=dev)
-        torch.cumsum(cnt.to(torch.int64), 0, out=off[1:])
-        return off
-
-    out = {"trace_idx": v["trace_local"].to(torch.int64) + trace_base, "occ_off": offsets(v["occ_cnt"], n_tr),
-           "ev_off": offsets(v["ev_cnt"], n_occ), "ev_pos": v["ev_pos"].to(torch.int32) & 0xFFFF,
-           "err_trace_idx": v["err_trace_idx"]}
-    if all_cols:
-        out["ev_rank"] = v["ev_rank"].to(torch.int32)
-        out["ev_act"] = v["ev_act"].to(torch.int32) & 0xFFFF
-        # event -> its trace: events per trace = sum of ev_cnt over the trace's occurrences
-        ev_per_occ = v["ev_cnt"].to(torch.int64)
-        occ_trace = torch.repeat_interleave(torch.arange(n_tr, device=dev), v["occ_cnt"].to(torch.int64))
-        ev_trace = torch.repeat_interleave(occ_trace, ev_per_occ)
-        out["ev_ts_ms"] = v["ts_base"][ev_trace] + v["ts_delta"].to(torch.int64) * (1000 if seconds else 1)
-    return out
-
-
-class JoinedMatches:
-    """The match lists of all ranks after exchange_blocks: parts[r] = dict of tensors (views into the receive buffer
-    for plain blocks, decoded columns for compact ones)."""
-
-    def __init__(self, recv, headers, work):
-        self.recv, self.headers, self._work = recv, headers, work
-        self.n_traces = int(sum(h[0] for h in headers))
-        self.n_occurrences = int(sum(h[1] for h in headers))
-        self.n_events = int(sum(h[2] for h in headers))
-
-    def wait(self):
-        """Block the current stream (not the host) until the all-gather has delivered every part."""
-        if self._work is not None:
-            self._work.wait()
-            self._work = None
-        return self
-
-    @property
-    def parts(self):
-        self.wait()
-        out = []
-        for r, h in enumerate(self.headers):
-            n_tr, n_occ, n_ev, n_err, all_cols, fmt = h[:6]
-            row = self.recv[r]
-            if fmt == 1:
-                out.append(unpack_block(row, h))
-            else:
-                lay, _ = block_layout(n_tr, n_occ, n_ev, n_err, all_cols)
-                out.append({k: row[o:o + nb].view(_DT[k]) for k, (o, nb) in lay.items()})
-        return out
-
-    def concatenated(self):
-        """One CSR over all ranks (copies; for consumers that want a single array per column)."""
-        parts = self.parts
-        out = {"trace_idx": torch.cat([p["trace_idx"] for p in parts]),
-               "err_trace_idx": torch.cat([p["err_trace_idx"] for p in parts])}
-        for name in ("occ_off", "ev_off"):
-            c = torch.cat([p[name][1:] - p[name][:-1] for p in parts])
-            off = torch.zeros(c.numel() + 1, dtype=torch.int64, device=c.device)
-            torch.cumsum(c, 0, out=off[1:])
-            out[name] = off
-        for k in ("ev_pos", "ev_rank", "ev_act", "ev_ts_ms"):
-            if k in parts[0]:
-                out[k] = torch.cat([p[k] for p in parts])
-        return out
-
-
-def exchange_blocks(block, header, group=None, async_op=True):
-    """All-gather of result blocks.  block: uint8 tensor; header: (n_traces, n_occurrences, n_events, n_ref_errors,
-    has_event_columns[, format, trace_base, seconds]) with format 0 = the library's plain block (DeviceMatches.block(),
-    pack_block()) and 1 = the compact wire format (DeviceMatches.packed_block()).  After this call returns the caller
-    may free `block` (it has been copied into the receive buffer); the all-gather itself may still be running."""
-    world = dist.get_world_size(group)
-    rank = dist.get_rank(group)
-    dev = block.device
-    header = (list(header) + [0, 0, 0])[:8]
-    h = torch.tensor(header + [block.numel()], dtype=torch.int64, device=dev)
-    hs = torch.empty(world * 9, dtype=torch.int64, device=dev)
-    if dev.type == "cuda":
-        dist.all_gather_into_tensor(hs, h, group=group)
-    else:
-        parts = [torch.empty_like(h) for _ in range(world)]
-        dist.all_gather(parts, h, group=group)
-        hs = torch.cat(parts)
-    hs = hs.view(world, 9).cpu().tolist()          # the only host synchronisation of the exchange
-    maxb = max(max(x[8] for x in hs), 256)
-    recv = torch.empty((world, maxb), dtype=torch.uint8, device=dev)
-    recv[rank, :block.numel()].copy_(block)
-    work = None
-    if dev.type == "cuda":
-        torch.cuda.current_stream(dev).synchronize()  # the copy is done: `block` may be freed by the caller
-        work = dist.all_gather_into_tensor(recv.view(-1), recv[rank], group=group, async_op=async_op)
-        if not async_op:
-            work = None
-    else:
-        rows = [torch.empty(maxb, dtype=torch.uint8) for _ in range(world)]
-        dist.all_gather(rows, recv[rank].clone(), group=group)
-        for r in range(world):
-            recv[r].copy_(rows[r])
-    return JoinedMatches(recv, [tuple(x[:8]) for x in hs], work)
-
-
-class PeerExchanger:
-    """exchange_blocks with the payload moved by the copy engines over NVLink peer memory instead of an SM-based NCCL
-    kernel: every rank stages its block in a symmetric-memory buffer and PULLS the other ranks' blocks with plain
-    device-to-device copies on a side stream (the pattern of torch's low-contention all-gather).  The copies use no SM,
-    so the next request's verification kernel runs beside them at full speed; only the 9-value header still goes
-    through NCCL.  One node only (symmetric memory needs peer access); `depth` requests may be in flight."""
-
-    def __init__(self, device, group=None, capacity=64 << 20, depth=3, n_streams=4):
-        import torch.distributed._symmetric_memory as symm
-        self._symm = symm
-        self.group = group if group is not None else dist.group.WORLD
-        self.device, self.depth = device, depth
-        self.rank, self.world = dist.get_rank(self.group), dist.get_world_size(self.group)
-        self.stream = torch.cuda.Stream(device)
-        # one copy engine does not fill an NVLink port: the pulls of one request are spread over several streams
-        self.pull_streams = [torch.cuda.Stream(device) for _ in range(max(1, int(os.environ.get("SIESTA_PEER_STREAMS", n_streams))))]
-        self.k = 0
-        self._alloc(capacity)
-
-    def _alloc(self, capacity):
-        self.capacity = int(capacity)
-        self.bufs = [self._symm.empty(self.capacity, dtype=torch.uint8, device=self.device) for _ in range(self.depth)]
-        self.hdls = [self._symm.rendezvous(b, self.group) for b in self.bufs]
-        self.free = [None] * self.depth   # event: every rank has finished pulling from this slot
-
-    def exchange(self, block, header):
-        """Same contract as exchange_blocks: on return `block` may be freed; the pulls may still be running."""
-        world, rank, dev = self.world, self.rank, self.device
-        header = (list(header) + [0, 0, 0])[:8]
-        h = torch.tensor(header + [block.numel()], dtype=torch.int64, device=dev)
-        hs = torch.empty(world * 9, dtype=torch.int64, device=dev)
-        dist.all_gather_into_tensor(hs, h, group=self.group)
-        hs = hs.view(world, 9).cpu().tolist()
-        maxb = max(max(x[8] for x in hs), 256)
-        if maxb > self.capacity:            # every rank sees the same sizes: a collective, deterministic decision
-            torch.cuda.synchronize(dev)
-            self._alloc(max(2 * maxb, 2 * self.capacity))
-        slot = self.k % self.depth
-        self.k += 1
-        cur = torch.cuda.current_stream(dev)
-        if self.free[slot] is not None:
-            cur.wait_event(self.free[slot])
-        self.bufs[slot][:block.numel()].copy_(block)
-        cur.synchronize()                    # the own block is staged: the caller may free it
-        recv = torch.empty((world, maxb), dtype=torch.uint8, device=dev)
-        hdl = self.hdls[slot]
-        self.stream.wait_stream(cur)
-        with torch.cuda.stream(self.stream):
-            hdl.barrier()                    # every rank has staged its block
-            staged = torch.cuda.Event()
-            staged.record(self.stream)
-        for step in range(world):
-            r = (rank - step) % world
-            n = hs[r][8]
-            if n:
-                st = self.pull_streams[step % len(self.pull_streams)]
-                st.wait_event(staged)
-                with torch.cuda.stream(st):
-                    src = hdl.get_buffer(r, (self.capacity,), torch.uint8)
-                    recv[r, :n].copy_(src[:n], non_blocking=True)
-        for st in self.pull_streams:
-            self.stream.wait_stream(st)
-            recv.record_stream(st)
-        with torch.cuda.stream(self.stream):
-            hdl.barrier()                    # every rank has pulled: the slot may be overwritten
-            done = torch.cuda.Event()
-            done.record(self.stream)
-        self.free[slot] = done
-        recv.record_stream(self.stream)
-        return JoinedMatches(recv, [tuple(x[:8]) for x in hs], _EventWork(done))
-
-
-class _EventWork:
-    def __init__(self, event):
-        self.event = event
-
-    def wait(self):
-        torch.cuda.current_stream().wait_event(self.event)
-
-
-def pack_block(tensors):
-    """dict of 1-D tensors (as DeviceMatches.tensors() / match_result_to_tensors) -> (uint8 block, header): the layout
-    the library produces natively; used where the result did not come from the library (CPU tests)."""
-    n_tr, n_occ = tensors["trace_idx"].numel(), tensors["ev_off"].numel() - 1
-    n_ev, n_err = tensors["ev_pos"].numel(), tensors["err_trace_idx"].numel()
-    all_cols = 1 if tensors.get("ev_rank") is not None else 0
-    lay, total = block_layout(n_tr, n_occ, n_ev, n_err, all_cols)
-    block = torch.zeros(max(total, 1), dtype=torch.uint8, device=tensors["trace_idx"].device)
-    for k, (o, nb) in lay.items():
-        if nb:
-            block[o:o + nb].copy_(tensors[k].contiguous().view(torch.uint8))
-    return block, (n_tr, n_occ, n_ev, n_err, all_cols)
 
 
 def allreduce_counts(packed, group=None):
@@ -354,13 +69,6 @@ def pair_stats_records(packed):
         sq = r[4] | (r[5] << 32) | (r[6] << 64) | (r[7] << 96)
         out.append({"count": cnt, "sum": r[1], "min": r[2] if cnt else 0, "max": r[3] if cnt else 0, "sum_squares": sq})
     return out
-
-
-def allreduce_explore(completions, sum_duration_ms, group=None):
-    """Combine siesta_explore_accurate results across ranks (both are plain sums over traces)."""
-    dist.all_reduce(completions, op=dist.ReduceOp.SUM, group=group)
-    dist.all_reduce(sum_duration_ms, op=dist.ReduceOp.SUM, group=group)
-    return completions, sum_duration_ms
 
 
 # ------------------------------------------------------------------------------------- exchange inside the library
@@ -438,6 +146,8 @@ def joined_prefix(tensors, n_first_traces):
 
 
 _COLS = ("trace_idx", "occ_off", "ev_off", "err_trace_idx", "ev_pos", "ev_rank", "ev_act", "ev_ts_ms")
+_DT = {"trace_idx": torch.int64, "occ_off": torch.int64, "ev_off": torch.int64, "ev_pos": torch.int32,
+       "err_trace_idx": torch.int64, "ev_rank": torch.int32, "ev_act": torch.int32, "ev_ts_ms": torch.int64}
 
 
 def send_columns(cols, dst, group=None):
@@ -477,9 +187,3 @@ def to_match_result(g, n_matches_emitted=-1):
     r.n_unsupported = len(r.unsupported_trace_idx)
     return r
 
-
-def match_result_to_tensors(res, device="cpu"):
-    d = {k: torch.from_numpy(np.ascontiguousarray(getattr(res, k))).to(device)
-         for k in ("trace_idx", "occ_off", "ev_off", "ev_pos", "ev_rank", "ev_act", "ev_ts_ms", "err_trace_idx")
-         if getattr(res, k) is not None}
-    return d

@@ -1,6 +1,7 @@
 """Worker of tests/test_distributed_cpu.py: launched by torch.distributed.run with the gloo backend on CPU.
-Each rank computes its shard with the ORACLE (test infrastructure standing in for the GPU kernels, which need a
-device), then runs the product's exchange code; rank 0 compares with the unsharded oracle result."""
+Each rank computes the counts of its shard with the ORACLE (test infrastructure standing in for the GPU kernels, which
+need a device), then combines them with the product's all-reduce code; rank 0 compares with the unsharded oracle
+result."""
 import json
 import os
 import sys
@@ -12,7 +13,6 @@ import torch.distributed as dist
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
 sys.path.insert(0, ROOT)
 import oracle  # noqa: E402
-from sequencedetectionqueryexecutor_b200 import _abi as abi  # noqa: E402
 from sequencedetectionqueryexecutor_b200 import distributed as D  # noqa: E402
 from tests import gen  # noqa: E402
 
@@ -21,23 +21,7 @@ def main():
     dist.init_process_group("gloo")
     rank, world = dist.get_rank(), dist.get_world_size()
     off, act, ts = gen.make_log(1500, 0, 40, 8, seed=2024)
-    nfa = abi.make_nfa([dict(kind=abi.STATE_NORMAL, types=[0]), dict(kind=abi.STATE_KLEENE_PLUS, types=[1]),
-                        dict(kind=abi.STATE_NORMAL, types=[2], preds=[(abi.ATTR_TIMESTAMP, abi.OP_LE, 0, 3000)])])
-    flags = abi.F_RETURN_ALL
-    l_off, l_act, l_ts, first = D.local_shard(off, act, ts, rank, world)
-    local = oracle.detect(l_off, l_act, l_ts, nfa, flags=flags)
-    g = D.allgather_matches(D.match_result_to_tensors(local), first)
-    got = D.to_match_result(g)
-    want = oracle.detect(off, act, ts, nfa, flags=flags)
-    ok_detect, why = got.same_as(want)
-    # the block exchange (one padded all-gather of the library's result block): same joined result
-    lt = D.match_result_to_tensors(local)
-    lt["trace_idx"] = lt["trace_idx"] + first        # what siesta_log_set_first_trace makes the library return
-    lt["err_trace_idx"] = lt["err_trace_idx"] + first
-    joined = D.exchange_blocks(*D.pack_block(lt))
-    ok_block, why_b = D.to_match_result(joined.concatenated()).same_as(want)
-    ok_detect = ok_detect and ok_block and joined.n_traces == want.n_traces
-    why = why or why_b
+    l_off, l_act = D.local_shard(off, act, ts, rank, world)[:2]
     lc = oracle.declare_counts(l_off, l_act, 8, 40)
     packed = D.allreduce_counts(torch.from_numpy(lc.packed.copy()))
     wc = oracle.declare_counts(off, act, 8, 40)
@@ -62,8 +46,8 @@ def main():
     ev = [int(off[b[r + 1]] - off[b[r]]) for r in range(world)]
     if rank == 0:
         with open(sys.argv[1], "w") as f:
-            json.dump({"ok_detect": bool(ok_detect), "why": why, "ok_declare": ok_declare, "ok_stats": bool(ok_stats), "world": world,
-                       "bounds": [int(x) for x in b], "events_per_rank": ev, "n_traces": int(want.n_traces)}, f)
+            json.dump({"ok_declare": ok_declare, "ok_stats": bool(ok_stats), "world": world,
+                       "bounds": [int(x) for x in b], "events_per_rank": ev}, f)
     dist.destroy_process_group()
 
 

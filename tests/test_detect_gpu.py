@@ -408,69 +408,43 @@ def test_explore_accurate_matches_per_candidate_detection(ctx):
         log.close()
 
 
-def test_result_block_and_shard_offsets(ctx):
-    """The device result is one allocation with a documented layout (shipped whole by the multi-GPU exchange), and a
-    log marked as a shard returns global trace indices."""
-    import torch
-    from sequencedetectionqueryexecutor_b200 import distributed as D
+def _block_layout(n_tr, n_occ, n_ev, n_err, n_unsup, all_cols):
+    """Byte offsets of the result columns inside siesta_dev_matches.d_block, in the order include/siesta_gpu.h
+    documents (each at a 256-byte aligned offset), and the block's size."""
+    cols = [("trace_idx", n_tr * 8), ("occ_off", (n_tr + 1) * 8), ("ev_off", (n_occ + 1) * 8), ("ev_pos", n_ev * 4),
+            ("err_trace_idx", n_err * 8)]
+    if all_cols:
+        cols += [("ev_rank", n_ev * 4), ("ev_act", n_ev * 4), ("ev_ts_ms", n_ev * 8)]
+    cols.append(("unsupported_trace_idx", n_unsup * 8))
+    off, o = {}, 0
+    for name, nbytes in cols:
+        off[name] = o
+        o += (nbytes + 255) & ~255
+    return off, o
+
+
+def test_result_block_layout_and_shard_offsets(ctx):
+    """The device result is one allocation with a documented layout, and a log marked as a shard returns global
+    trace indices."""
     off, act, ts = gen.make_log(3000, 0, 40, 8, seed=91)
     nfa = abi.make_nfa([dict(kind=X_, types=[3]), dict(kind=N_, types=[0]), dict(kind=P_, types=[1]), dict(kind=N_, types=[2])])
     want = oracle.detect(off, act, ts, nfa, flags=abi.F_RETURN_ALL)
     log = ctx.load_log(off, act, ts, 8)
     log.set_first_trace(1_000_000)
     dm = log.detect_device(nfa, flags=abi.F_RETURN_ALL)
-    block, header = dm.block(0)
-    lay, total = D.block_layout(*header)
-    assert total == block.numel() and header[:4] == (want.n_traces, want.n_occurrences, want.n_events, want.n_ref_errors)
-    views = {k: block[o:o + nb].view(D._DT[k]).cpu().numpy() for k, (o, nb) in lay.items()}
-    torch.cuda.synchronize()
-    assert np.array_equal(views["trace_idx"], want.trace_idx + 1_000_000)
-    assert np.array_equal(views["err_trace_idx"], want.err_trace_idx + 1_000_000)
+    d = dm.dm
+    assert (d.n_traces, d.n_occurrences, d.n_events, d.n_ref_errors) == (want.n_traces, want.n_occurrences, want.n_events, want.n_ref_errors)
+    lay, total = _block_layout(d.n_traces, d.n_occurrences, d.n_events, d.n_ref_errors, d.n_unsupported, d.d_ev_rank)
+    assert total == d.block_bytes
+    for k, o in lay.items():
+        assert getattr(d, "d_" + k) == d.d_block + o, k
+    got = {k: v.cpu().numpy() for k, v in dm.tensors(0).items()}
+    assert np.array_equal(got["trace_idx"], want.trace_idx + 1_000_000)
+    assert np.array_equal(got["err_trace_idx"], want.err_trace_idx + 1_000_000)
     for k in ("occ_off", "ev_off", "ev_pos", "ev_rank", "ev_act", "ev_ts_ms"):
-        assert np.array_equal(views[k], getattr(want, k)), k
+        assert np.array_equal(got[k], getattr(want, k)), k
     dm.close()
     log.close()
-
-
-def test_compact_wire_format_round_trip(ctx):
-    """siesta_dev_matches_pack + distributed.unpack_block reproduce every column of the device result (EventTs and
-    EventPos routes, returnAll, reference-throw traces); values that do not fit are refused, not truncated."""
-    import torch
-    from sequencedetectionqueryexecutor_b200 import distributed as D
-    off, act, ts = gen.make_log(4000, 0, 50, 8, seed=93, jitter_ms=True)
-    cases = [([dict(kind=P_, types=[0]), dict(kind=S_, types=[1], preds=[(abi.ATTR_TIMESTAMP, abi.OP_LE, 0, 900)])], 0),
-             ([dict(kind=N_, types=[0]), dict(kind=P_, types=[1]), dict(kind=N_, types=[2])], abi.F_RETURN_ALL),
-             ([dict(kind=N_, types=[0]), dict(kind=N_, types=[1])], abi.F_EVT_POS | abi.F_RETURN_ALL),
-             ([dict(kind=X_, types=[1]), dict(kind=P_, types=[2])], 0)]
-    log = ctx.load_log(off, act, ts, 8)
-    log.set_first_trace(7_000_000_000)
-    try:
-        for states, flags in cases:
-            dm = log.detect_device(abi.make_nfa(states), flags=flags)
-            want = {k: v.clone() for k, v in dm.tensors(0).items()}
-            packed = dm.packed_block(log, flags, 7_000_000_000, 0)
-            assert packed is not None
-            block, header = packed
-            plain, _ = dm.block(0)
-            assert block.numel() < 0.6 * plain.numel() or dm.n_events < 20_000  # small results are all alignment padding
-            got = D.unpack_block(block, header)
-            torch.cuda.synchronize()
-            for k, v in want.items():
-                if k != "unsupported_trace_idx":   # (not part of this older wire format; siesta_detect_allgather ships it)
-                    assert torch.equal(got[k], v), (k, states, flags)
-            dm.close()
-    finally:
-        log.close()
-    # an activity id beyond 65 535 does not fit ev_act: the pack call refuses, the plain block is shipped instead
-    off2, act2, ts2 = gen.make_log(50, 10, 20, 5, seed=94)
-    act2 = act2.copy()
-    act2[act2 == 0] = 66_000
-    act2[act2 == 1] = 66_001
-    log2 = ctx.load_log(off2, act2, ts2, 70_000)
-    dm = log2.detect_device(abi.make_nfa([dict(kind=N_, types=[66_000]), dict(kind=N_, types=[66_001])]), flags=0)
-    assert dm.n_traces >= 1 and dm.packed_block(log2, 0, 0, 0) is None
-    dm.close()
-    log2.close()
 
 
 def test_concurrent_requests_on_one_log(ctx):
