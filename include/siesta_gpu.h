@@ -456,6 +456,36 @@ int siesta_index_load(siesta_log* log, int32_t n_pairs, const int32_t* pair_a, c
  * (A,B) iff it holds an A before a B (A == B: at least two occurrences).  <= 32 pairs / 32 distinct activities. */
 int siesta_index_build(siesta_log* log, const int32_t* pair_a, const int32_t* pair_b, int32_t n_pairs,
                        siesta_index** out);
+/* After siesta_log_append: a new index on new_log (the log the append returned, or one grown from it by later appends)
+ * that follows the appended events.  Neither call modifies `index`: it stays valid on its own log and keeps answering
+ * siesta_intersect / siesta_candidates while the new one is built; the caller swaps handles as with the log.  `index`'s log
+ * must still be alive during the call.  Both are exact because an append only adds events after a trace's existing ones:
+ * a trace keeps every pair it held, so no trace leaves a list, and traces the batch did not list are unchanged.
+ * SIESTA_E_INVALID (nothing allocated, *out untouched, `index` unchanged): a null argument, new_log on another context or
+ * with fewer traces than the index's log, or the call-specific cases below.  *kernel_ms (may be NULL) = device time between
+ * CUDA events on the context's stream after the host -> device copies (work other threads enqueue on the context during
+ * the call is counted too).
+ *
+ * siesta_index_append: list p = index's list p UNION delta list p (ascending, duplicate-free).  Delta list p =
+ * delta_trace_idx[delta_off[p] .. delta_off[p+1]), strictly ascending trace indices of new_log, in the index's pair order;
+ * it may repeat traces the old list holds (index.parquet rows of a batch name traces that were listed before).
+ * delta_trace_idx may be NULL when every delta list is empty.  The result counts as a loaded index, whatever `index` was.
+ * Refused: delta_off[0] != 0, delta_off decreasing, a delta list not strictly ascending or holding an index outside
+ * [0, new_log's n_traces). */
+int siesta_index_append(siesta_index* index, siesta_log* new_log, const int64_t* delta_off, const int64_t* delta_trace_idx,
+                        siesta_index** out, double* kernel_ms);
+/* siesta_index_refresh: built indexes only (siesta_index_build or an earlier refresh).  Re-derives, under the SeqTable
+ * view on new_log, the membership of the traces the batch listed (trace_idx[n_listed] exactly as passed to
+ * siesta_log_append, strictly ascending; NULL when n_listed == 0) and merges it into the old lists: the result equals
+ * siesta_index_build(new_log, same pairs) and is a built index.  One case re-flags EVERY trace: when the index's log held
+ * activity ids outside its alphabet (not every id of the log lies in [0, n_activities)) and new_log's larger alphabet
+ * covers an activity one of the pairs names, unlisted traces that hold such an id gain the pair, as
+ * siesta_index_build counts them now; the call then costs a full build.  Refused: a loaded index (siesta_index_load or
+ * siesta_index_append), n_listed < 0, trace_idx not strictly ascending or outside [0, new_log's n_traces), or not
+ * listing every new trace [index's n_traces, new_log's n_traces).  SIESTA_E_UNSUPPORTED as siesta_index_build when the
+ * pairs mention more than 32 activities of new_log's alphabet. */
+int siesta_index_refresh(siesta_index* index, siesta_log* new_log, const int64_t* trace_idx, int64_t n_listed,
+                         siesta_index** out, double* kernel_ms);
 void siesta_index_free(siesta_index* index);
 int64_t siesta_index_list_len(const siesta_index* index, int32_t pair);
 int siesta_index_get_list(const siesta_index* index, int32_t pair, int64_t* out, int64_t cap);

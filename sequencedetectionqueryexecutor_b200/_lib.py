@@ -24,7 +24,7 @@ EXPORTS = [
     "siesta_multi_init", "siesta_multi_shutdown", "siesta_multi_n_devices", "siesta_multi_log_load", "siesta_multi_log_free",
     "siesta_multi_log_shard", "siesta_multi_detect", "siesta_multi_declare_counts", "siesta_multi_why_not_match",
     "siesta_log_filter_time", "siesta_log_group", "siesta_log_source_events",
-    "siesta_log_append", "siesta_log_read", "siesta_multi_log_append",
+    "siesta_log_append", "siesta_log_read", "siesta_multi_log_append", "siesta_index_append", "siesta_index_refresh",
 ]
 
 
@@ -77,6 +77,8 @@ def lib():
     L.siesta_declare_counts_device.argtypes = [vp, i32, vp, vp, P(C.c_double)]
     L.siesta_index_load.argtypes = [vp, i32, vp, vp, vp, vp, P(vp)]
     L.siesta_index_build.argtypes = [vp, vp, vp, i32, P(vp)]
+    L.siesta_index_append.argtypes = [vp, vp, vp, vp, P(vp), P(C.c_double)]
+    L.siesta_index_refresh.argtypes = [vp, vp, vp, i64, P(vp), P(C.c_double)]
     L.siesta_index_free.argtypes = [vp]
     L.siesta_index_free.restype = None
     L.siesta_index_list_len.argtypes = [vp, i32]

@@ -275,6 +275,15 @@ class EventLog:
         return PairIndex(self, pairs, lists=lists)
 
 
+def _flat_lists(lists):
+    """Posting lists back to back as the C-ABI takes them: (offsets int64[n + 1], entries int64)."""
+    lists = [np.ascontiguousarray(x, dtype=np.int64) for x in lists]
+    off = np.zeros(len(lists) + 1, dtype=np.int64)
+    np.cumsum([len(x) for x in lists], out=off[1:])
+    flat = np.concatenate(lists) if lists and off[-1] else np.zeros(0, dtype=np.int64)
+    return off, flat
+
+
 class PairIndex:
     """siesta_index: per-pair posting lists in HBM + the sorted trace-id intersection (kernel K2)."""
 
@@ -287,11 +296,34 @@ class PairIndex:
         if lists is None:
             check(lib().siesta_index_build(log._h, _ptr(pa), _ptr(pb), len(self.pairs), C.byref(self._h)))
         else:
-            lists = [np.ascontiguousarray(x, dtype=np.int64) for x in lists]
-            off = np.zeros(len(lists) + 1, dtype=np.int64)
-            np.cumsum([len(x) for x in lists], out=off[1:])
-            flat = np.concatenate(lists) if lists and off[-1] else np.zeros(0, dtype=np.int64)
+            off, flat = _flat_lists(lists)
             check(lib().siesta_index_load(log._h, len(self.pairs), _ptr(pa), _ptr(pb), _ptr(off), _ptr(flat), C.byref(self._h)))
+
+    def _adopt(self, new_log, h):
+        out = PairIndex.__new__(PairIndex)
+        out.log, out.pairs, out._h = new_log, list(self.pairs), h
+        return out
+
+    def append(self, new_log, lists):
+        """siesta_index_append: a new index on new_log (this log with batches appended) whose list p = this list p UNION
+        lists[p] (ascending trace indices of new_log, aligned with self.pairs; an empty array leaves the pair as it is),
+        e.g. a batch's index.parquet rows read by ingest.read_index_table -> (PairIndex, kernel_ms).  This index is not
+        modified and stays usable; the result counts as loaded lists."""
+        if len(lists) != len(self.pairs):
+            raise ValueError(f"{len(lists)} delta lists for an index of {len(self.pairs)} pairs")
+        off, flat = _flat_lists(lists)
+        h, ms = C.c_void_p(), C.c_double(0.0)
+        check(lib().siesta_index_append(self._h, new_log._h, _ptr(off), _ptr(flat), C.byref(h), C.byref(ms)))
+        return self._adopt(new_log, h), ms.value
+
+    def refresh(self, new_log, trace_idx):
+        """siesta_index_refresh (built indexes only): re-derive the traces a log append listed (trace_idx as passed to
+        EventLog.append) on new_log and merge -> (PairIndex equal to new_log.build_index(self.pairs), kernel_ms).  This
+        index is not modified and stays usable."""
+        ti = np.ascontiguousarray(trace_idx, dtype=np.int64)
+        h, ms = C.c_void_p(), C.c_double(0.0)
+        check(lib().siesta_index_refresh(self._h, new_log._h, _ptr(ti) if len(ti) else None, len(ti), C.byref(h), C.byref(ms)))
+        return self._adopt(new_log, h), ms.value
 
     def close(self):
         if self._h:

@@ -18,7 +18,6 @@
 
 namespace siesta {
 
-constexpr int AP_T = 256;           // threads per block
 constexpr int64_t AP_TILE = 8192;   // output events per block of the copy kernel
 
 // One thread per trace of the new log (and one for the closing offset): new_off[t] = old_off[min(t, T)] + batch_off[j]
@@ -50,28 +49,6 @@ __global__ void __launch_bounds__(AP_T) ap_offsets_kernel(const int64_t* __restr
 #pragma unroll
     for (int d = 16; d; d >>= 1) len = max(len, __shfl_xor_sync(0xffffffffu, len, d));
     if ((threadIdx.x & 31) == 0 && len) atomicMax(max_len, len);
-}
-
-// Block-wide copy of n elements.  16-byte loads and stores when source and destination agree modulo 16 bytes (scalar
-// head and tail), coalesced element copies otherwise.
-template <typename T>
-__device__ __forceinline__ void ap_copy(T* __restrict__ dst, const T* __restrict__ src, int64_t n) {
-    constexpr int V = 16 / sizeof(T);
-    if ((((uintptr_t)dst ^ (uintptr_t)src) & 15) == 0) {
-        int64_t head = (int64_t)(((16 - ((uintptr_t)dst & 15)) & 15) / sizeof(T));
-        head = head < n ? head : n;
-        if (threadIdx.x < head) dst[threadIdx.x] = src[threadIdx.x];
-        const int64_t nv = (n - head) / V;
-        int4* __restrict__ dv = reinterpret_cast<int4*>(dst + head);
-        const int4* __restrict__ sv = reinterpret_cast<const int4*>(src + head);
-#pragma unroll 4
-        for (int64_t i = threadIdx.x; i < nv; i += AP_T) dv[i] = __ldg(sv + i);
-        const int64_t done = head + nv * V;
-        if (done + threadIdx.x < n) dst[done + threadIdx.x] = src[done + threadIdx.x];
-    } else {
-#pragma unroll 8
-        for (int64_t i = threadIdx.x; i < n; i += AP_T) dst[i] = __ldg(src + i);
-    }
 }
 
 // Grid over the output columns, AP_TILE events per block.  The block finds the first piece that reaches into its tile

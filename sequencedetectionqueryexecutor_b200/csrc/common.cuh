@@ -36,6 +36,31 @@ extern std::atomic<long long> g_kernel_launches;
 
 #define SIESTA_LAUNCHED() (::siesta::g_kernel_launches.fetch_add(1, std::memory_order_relaxed))
 
+// Block-wide copy of n elements by blocks of AP_T threads (append.cu, intersect.cu).  16-byte loads and stores when
+// source and destination agree modulo 16 bytes (scalar head and tail), coalesced element copies otherwise.
+constexpr int AP_T = 256;
+#ifdef __CUDACC__
+template <typename T>
+__device__ __forceinline__ void ap_copy(T* __restrict__ dst, const T* __restrict__ src, int64_t n) {
+    constexpr int V = 16 / sizeof(T);
+    if ((((uintptr_t)dst ^ (uintptr_t)src) & 15) == 0) {
+        int64_t head = (int64_t)(((16 - ((uintptr_t)dst & 15)) & 15) / sizeof(T));
+        head = head < n ? head : n;
+        if (threadIdx.x < head) dst[threadIdx.x] = src[threadIdx.x];
+        const int64_t nv = (n - head) / V;
+        int4* __restrict__ dv = reinterpret_cast<int4*>(dst + head);
+        const int4* __restrict__ sv = reinterpret_cast<const int4*>(src + head);
+#pragma unroll 4
+        for (int64_t i = threadIdx.x; i < nv; i += AP_T) dv[i] = __ldg(sv + i);
+        const int64_t done = head + nv * V;
+        if (done + threadIdx.x < n) dst[done + threadIdx.x] = src[done + threadIdx.x];
+    } else {
+#pragma unroll 8
+        for (int64_t i = threadIdx.x; i < n; i += AP_T) dst[i] = __ldg(src + i);
+    }
+}
+#endif
+
 // Pinned host blocks that result objects (siesta_matches) are carved from; blocks return here on siesta_matches_free
 // and are reused by later calls, so a steady-state request pays no cudaHostAlloc.
 struct HostBlock {

@@ -13,6 +13,10 @@
 //                       the intersection of n duplicate-free lists iff its counter reaches n: every list is read
 //                       exactly once, coalesced (8 B x sum |list_i|), no search
 //   compaction          block counts -> one-block scan -> ordered write (ascending output, deterministic)
+//   index_dup_kernel    one thread per element of the delta lists of an index refresh / append: rank in its old list (one
+//                       binary search) and whether the old list holds it already
+//   index_merge_kernel  grid over the merged lists: runs of old entries, each shifted by the inserts before it, and the
+//                       groups of inserts between them, copied as contiguous pieces
 #include <algorithm>
 #include <cstring>
 #include <vector>
@@ -30,6 +34,7 @@ struct Index {
     std::vector<int32_t> pair_a, pair_b;
     std::vector<int64_t> off;       // [n_pairs + 1] into d_lists
     int64_t* d_lists = nullptr;     // all posting lists back to back (device)
+    bool built = false;             // siesta_index_build / siesta_index_refresh (SeqTable view), not loaded lists
 };
 
 // ------------------------------------------------------------------------------------------------ compaction
@@ -107,7 +112,8 @@ __global__ void __launch_bounds__(IT) flag_write_kernel(const uint8_t* flags, co
 struct PairFlagParams {
     const int64_t* trace_off;
     const int32_t* act;
-    int64_t n_traces;
+    const int64_t* work;    // nullptr: row t is trace t; else row i is trace work[i]
+    int64_t n_traces;       // rows: the log's traces, or the entries of work
     const int8_t* slot_of;  // [n_act] activity -> scratch slot (0..31) or -1
     int32_t n_act;
     int32_t n_pairs;
@@ -120,7 +126,8 @@ __global__ void __launch_bounds__(IT) pair_flags_kernel(const __grid_constant__ 
     const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
     const long long warps_total = (long long)gridDim.x * (IT / 32);
     for (long long t = (long long)blockIdx.x * (IT / 32) + warp; t < P.n_traces; t += warps_total) {
-        const long long lo = P.trace_off[t], hi = P.trace_off[t + 1];
+        const long long tr = P.work ? P.work[t] : t;
+        const long long lo = P.trace_off[tr], hi = P.trace_off[tr + 1];
         s_cnt[warp][lane] = 0;
         s_first[warp][lane] = 0xffffffffu;
         s_last[warp][lane] = 0;
@@ -229,6 +236,206 @@ static int compact_rows(cudaStream_t stream, const uint8_t* d_flags, const int64
     return SIESTA_OK;
 }
 
+// Posting lists of the pairs under the SeqTable view over every trace of L (d_work == nullptr) or over the n_work
+// ascending traces d_work lists: list p = row_off[p] .. row_off[p + 1]) of *d_lists, ascending trace indices.
+static int build_lists(const char* fn, Log* L, const int32_t* pair_a, const int32_t* pair_b, int32_t n_pairs, const int64_t* d_work,
+                       int64_t n_work, std::vector<int64_t>& row_off, int64_t** d_lists) {
+    cudaStream_t stream = L->ctx->stream;
+    // activities mentioned by the pairs -> scratch slots
+    std::vector<int8_t> slot_of((size_t)std::max(1, L->n_activities), -1);
+    PairFlagParams P;
+    std::memset(&P, 0, sizeof(P));
+    int n_slots = 0;
+    auto slot = [&](int a) -> int {
+        if (a < 0 || a >= L->n_activities) return -1;  // activity unknown to the log: empty list
+        if (slot_of[a] < 0) slot_of[a] = (int8_t)n_slots++;
+        return slot_of[a];
+    };
+    for (int p = 0; p < n_pairs; ++p) {
+        P.slot_a[p] = (int8_t)slot(pair_a[p]);
+        P.slot_b[p] = (int8_t)slot(pair_b[p]);
+        if (n_slots > 32) {
+            set_error(std::string(fn) + ": the pairs of one call may mention at most 32 distinct activities");
+            return SIESTA_E_UNSUPPORTED;
+        }
+    }
+    const int64_t n = d_work ? n_work : L->n_traces;
+    int8_t* d_slot = nullptr;
+    uint8_t* d_flags = nullptr;
+    SIESTA_CUDA_OK(cudaMallocAsync((void**)&d_slot, slot_of.size(), stream));
+    SIESTA_CUDA_OK(cudaMallocAsync((void**)&d_flags, (size_t)std::max<int64_t>(n, 1) * n_pairs, stream));
+    SIESTA_CUDA_OK(cudaMemcpyAsync(d_slot, slot_of.data(), slot_of.size(), cudaMemcpyHostToDevice, stream));
+    P.trace_off = L->d_trace_off;
+    P.act = L->d_act;
+    P.work = d_work;
+    P.n_traces = n;
+    P.slot_of = d_slot;
+    P.n_act = L->n_activities;
+    P.n_pairs = n_pairs;
+    P.flags = d_flags;
+    if (n > 0) {
+        const int64_t ctas = (n + IT / 32 - 1) / (IT / 32);
+        const int grid = (int)std::min<int64_t>(ctas, (int64_t)L->ctx->sm_count * 8);
+        pair_flags_kernel<<<grid, IT, 0, stream>>>(P);
+        SIESTA_LAUNCHED();
+        SIESTA_CUDA_OK(cudaGetLastError());
+    }
+    std::vector<int64_t> counts;
+    int rc = compact_rows(stream, d_flags, d_work, n, n_pairs, counts, d_lists, row_off);
+    cudaFreeAsync(d_slot, stream);
+    cudaFreeAsync(d_flags, stream);
+    return rc;
+}
+
+// ------------------------------------------------------------------------------------------------ index merge
+// The old lists O (back to back) and the delta lists (back to back, same pair order) merge into one flat pass: a delta
+// element of pair p that O does not hold goes before O[R] with R = old_off[p] + (its rank in old list p).  Numbered in
+// delta order, the k-th such insert lands at R_k + k; R_k never decreases (pairs in order, ranks ascend inside a pair), so
+// the output is O cut at the R_k, old run k (between inserts k - 1 and k) shifted by k, with the inserts between the runs.
+constexpr int64_t IM_TILE = 8192;   // output entries per block of index_merge_kernel
+
+// One thread per delta element: R[i], nd[i] = 1 unless the old list holds the element, dup[p] += duplicates of pair p.
+__global__ void __launch_bounds__(IT) index_dup_kernel(const int64_t* __restrict__ delta, int64_t D, const int64_t* __restrict__ doff,
+                                                       int32_t n_pairs, const int64_t* __restrict__ old, const int64_t* __restrict__ ooff,
+                                                       int64_t* __restrict__ R, uint8_t* __restrict__ nd, unsigned long long* dup) {
+    const int64_t i = (int64_t)blockIdx.x * IT + threadIdx.x;
+    int p = 0;
+    bool is_dup = false;
+    if (i < D) {
+        int lo = 0, hi = n_pairs - 1;   // the pair whose delta range holds i: first p with doff[p + 1] > i
+        while (lo < hi) {
+            const int mid = (lo + hi) >> 1;
+            if (__ldg(doff + mid + 1) <= i) lo = mid + 1; else hi = mid;
+        }
+        p = lo;
+        const int64_t x = __ldg(delta + i), end = __ldg(ooff + p + 1);
+        int64_t a = __ldg(ooff + p), b = end;
+        if (a < b && __ldg(old + b - 1) < x) {
+            a = b;   // past the last old entry: every new trace lands here without a search
+        } else {
+            while (a < b) {
+                const int64_t mid = (a + b) >> 1;
+                if (__ldg(old + mid) < x) a = mid + 1; else b = mid;
+            }
+        }
+        is_dup = a < end && __ldg(old + a) == x;
+        R[i] = a;
+        nd[i] = is_dup ? 0 : 1;
+    }
+    const unsigned m = __ballot_sync(0xffffffffu, is_dup);
+    if (is_dup) {   // one atomic per pair and warp
+        const unsigned same = __match_any_sync(m, p);
+        if ((int)(threadIdx.x & 31) == __ffs(same) - 1) atomicAdd(dup + p, (unsigned long long)__popc(same));
+    }
+}
+
+// Grid over the N merged entries, IM_TILE per block; insert k (value ins[k]) sits at R[k] + k, strictly ascending.  The
+// block finds the first insert at or after its tile by binary search, then walks the pieces of the tile: old runs, and
+// groups of inserts that share R (no old entry between them) as one contiguous copy.
+__global__ void __launch_bounds__(AP_T) index_merge_kernel(const int64_t* __restrict__ old, const int64_t* __restrict__ R,
+                                                           const int64_t* __restrict__ ins, int64_t K, int64_t N, int64_t* __restrict__ out) {
+    const int64_t o0 = (int64_t)blockIdx.x * IM_TILE;
+    const int64_t o1 = o0 + IM_TILE < N ? o0 + IM_TILE : N;
+    int64_t lo = 0, hi = K;
+    while (lo < hi) {
+        const int64_t mid = (lo + hi) >> 1;
+        if (R[mid] + mid < o0) lo = mid + 1; else hi = mid;
+    }
+    int64_t i = lo, o = o0;   // o is an old entry before insert i, or insert i itself
+    while (o < o1) {
+        const int64_t d = i < K ? R[i] + i : N;   // old run i ends where insert i sits
+        if (o < d) {
+            const int64_t n = (d < o1 ? d : o1) - o;
+            ap_copy(out + o, old + (o - i), n);
+            o += n;
+        }
+        if (o >= o1 || i >= K) break;
+        const int64_t r = R[i];
+        int64_t a = i + 1, b = i + (o1 - o) < K ? i + (o1 - o) : K;   // inserts i .. j-1 share r; the tile holds o1 - o
+        while (a < b) {
+            const int64_t mid = (a + b) >> 1;
+            if (R[mid] == r) a = mid + 1; else b = mid;
+        }
+        const int64_t n = a - i;
+        ap_copy(out + o, ins + i, n);
+        o += n;
+        i = a;
+    }
+}
+
+// out list p = old list p UNION delta list p (both ascending, duplicate-free); delta lists on the device, offsets on the host.
+static int merge_lists(cudaStream_t stream, const int64_t* d_old, const std::vector<int64_t>& old_off, const int64_t* d_delta,
+                       const std::vector<int64_t>& doff, int32_t n_pairs, int64_t** d_out, std::vector<int64_t>& new_off) {
+    const int64_t D = doff[n_pairs], n_old = old_off[n_pairs];
+    std::vector<unsigned long long> h_dup((size_t)n_pairs, 0);
+    int64_t *d_doff = nullptr, *d_ooff = nullptr, *d_R = nullptr, *d_insR = nullptr, *d_insV = nullptr;
+    unsigned long long *d_dup = nullptr, *d_blk = nullptr, *d_cnt = nullptr;
+    uint8_t* d_nd = nullptr;
+    const int64_t n_blk = std::max<int64_t>((D + IT - 1) / IT, 1);
+    auto release = [&]() {
+        for (void* p : {(void*)d_doff, (void*)d_ooff, (void*)d_R, (void*)d_insR, (void*)d_insV, (void*)d_dup, (void*)d_blk, (void*)d_cnt, (void*)d_nd})
+            if (p) cudaFreeAsync(p, stream);
+    };
+    cudaError_t e = cudaSuccess;
+    auto A = [&](void** p, size_t bytes) {
+        if (e == cudaSuccess) e = cudaMallocAsync(p, std::max<size_t>(bytes, 8), stream);
+    };
+    A((void**)&d_doff, sizeof(int64_t) * (size_t)(n_pairs + 1));
+    A((void**)&d_ooff, sizeof(int64_t) * (size_t)(n_pairs + 1));
+    A((void**)&d_R, sizeof(int64_t) * (size_t)D);
+    A((void**)&d_insR, sizeof(int64_t) * (size_t)D);
+    A((void**)&d_insV, sizeof(int64_t) * (size_t)D);
+    A((void**)&d_nd, (size_t)D);
+    A((void**)&d_dup, sizeof(unsigned long long) * (size_t)n_pairs);
+    A((void**)&d_blk, sizeof(unsigned long long) * (size_t)n_blk);
+    A((void**)&d_cnt, sizeof(unsigned long long));
+    if (e == cudaSuccess) e = cudaMemcpyAsync(d_doff, doff.data(), sizeof(int64_t) * (size_t)(n_pairs + 1), cudaMemcpyHostToDevice, stream);
+    if (e == cudaSuccess) e = cudaMemcpyAsync(d_ooff, old_off.data(), sizeof(int64_t) * (size_t)(n_pairs + 1), cudaMemcpyHostToDevice, stream);
+    if (e == cudaSuccess) e = cudaMemsetAsync(d_dup, 0, sizeof(unsigned long long) * (size_t)n_pairs, stream);
+    if (e == cudaSuccess && D > 0) {
+        index_dup_kernel<<<(unsigned)n_blk, IT, 0, stream>>>(d_delta, D, d_doff, n_pairs, d_old, d_ooff, d_R, d_nd, d_dup);
+        SIESTA_LAUNCHED();
+        // inserts in delta order: their R and their values, compacted by the flag scan of the compaction
+        flag_count_kernel<<<(unsigned)n_blk, IT, 0, stream>>>(d_nd, D, n_blk, d_blk, 0);
+        SIESTA_LAUNCHED();
+        row_scan_kernel<<<1, 1024, 0, stream>>>(d_blk, n_blk, d_cnt);
+        SIESTA_LAUNCHED();
+        flag_write_kernel<<<(unsigned)n_blk, IT, 0, stream>>>(d_nd, d_R, D, n_blk, d_blk, nullptr, d_insR, 0);
+        SIESTA_LAUNCHED();
+        flag_write_kernel<<<(unsigned)n_blk, IT, 0, stream>>>(d_nd, d_delta, D, n_blk, d_blk, nullptr, d_insV, 0);
+        SIESTA_LAUNCHED();
+        e = cudaGetLastError();
+    }
+    if (e == cudaSuccess) e = cudaMemcpyAsync(h_dup.data(), d_dup, sizeof(unsigned long long) * (size_t)n_pairs, cudaMemcpyDeviceToHost, stream);
+    if (e == cudaSuccess) e = cudaStreamSynchronize(stream);
+    if (e != cudaSuccess) {
+        cudaGetLastError();
+        release();
+        set_error(std::string("index merge: ") + cudaGetErrorString(e));
+        return SIESTA_E_CUDA;
+    }
+    new_off.assign((size_t)n_pairs + 1, 0);
+    for (int p = 0; p < n_pairs; ++p)
+        new_off[p + 1] = new_off[p] + (old_off[p + 1] - old_off[p]) + (doff[p + 1] - doff[p]) - (int64_t)h_dup[p];
+    const int64_t N = new_off[n_pairs], K = N - n_old;
+    *d_out = nullptr;
+    e = cudaMallocAsync((void**)d_out, sizeof(int64_t) * (size_t)std::max<int64_t>(N, 1), stream);
+    if (e == cudaSuccess && N > 0) {
+        index_merge_kernel<<<(unsigned)((N + IM_TILE - 1) / IM_TILE), AP_T, 0, stream>>>(d_old, d_insR, d_insV, K, N, *d_out);
+        SIESTA_LAUNCHED();
+        e = cudaGetLastError();
+    }
+    release();
+    if (e != cudaSuccess) {
+        cudaGetLastError();
+        if (*d_out) cudaFreeAsync(*d_out, stream);
+        *d_out = nullptr;
+        set_error(std::string("index merge: ") + cudaGetErrorString(e));
+        return SIESTA_E_CUDA;
+    }
+    return SIESTA_OK;
+}
+
 }  // namespace siesta
 
 using namespace siesta;
@@ -245,54 +452,13 @@ extern "C" int siesta_index_build(siesta_log* log, const int32_t* pair_a, const 
     }
     Log* L = reinterpret_cast<Log*>(log);
     SIESTA_CUDA_OK(cudaSetDevice(L->ctx->device));
-    cudaStream_t stream = L->ctx->stream;
-    // activities mentioned by the pairs -> scratch slots
-    std::vector<int8_t> slot_of((size_t)std::max(1, L->n_activities), -1);
-    PairFlagParams P;
-    std::memset(&P, 0, sizeof(P));
-    int n_slots = 0;
-    auto slot = [&](int a) -> int {
-        if (a < 0 || a >= L->n_activities) return -1;  // activity unknown to the log: empty list
-        if (slot_of[a] < 0) slot_of[a] = (int8_t)n_slots++;
-        return slot_of[a];
-    };
-    for (int p = 0; p < n_pairs; ++p) {
-        P.slot_a[p] = (int8_t)slot(pair_a[p]);
-        P.slot_b[p] = (int8_t)slot(pair_b[p]);
-        if (n_slots > 32) {
-            set_error("siesta_index_build: the pairs of one call may mention at most 32 distinct activities");
-            return SIESTA_E_UNSUPPORTED;
-        }
-    }
-    const int64_t T = L->n_traces;
-    int8_t* d_slot = nullptr;
-    uint8_t* d_flags = nullptr;
-    SIESTA_CUDA_OK(cudaMallocAsync((void**)&d_slot, slot_of.size(), stream));
-    SIESTA_CUDA_OK(cudaMallocAsync((void**)&d_flags, (size_t)std::max<int64_t>(T, 1) * n_pairs, stream));
-    SIESTA_CUDA_OK(cudaMemcpyAsync(d_slot, slot_of.data(), slot_of.size(), cudaMemcpyHostToDevice, stream));
-    P.trace_off = L->d_trace_off;
-    P.act = L->d_act;
-    P.n_traces = T;
-    P.slot_of = d_slot;
-    P.n_act = L->n_activities;
-    P.n_pairs = n_pairs;
-    P.flags = d_flags;
-    if (T > 0) {
-        const int64_t ctas = (T + IT / 32 - 1) / (IT / 32);
-        const int grid = (int)std::min<int64_t>(ctas, (int64_t)L->ctx->sm_count * 8);
-        pair_flags_kernel<<<grid, IT, 0, stream>>>(P);
-        SIESTA_LAUNCHED();
-        SIESTA_CUDA_OK(cudaGetLastError());
-    }
     Index* ix = new Index();
     ix->log = L;
     ix->n_pairs = n_pairs;
     ix->pair_a.assign(pair_a, pair_a + n_pairs);
     ix->pair_b.assign(pair_b, pair_b + n_pairs);
-    std::vector<int64_t> counts;
-    int rc = compact_rows(stream, d_flags, nullptr, T, n_pairs, counts, &ix->d_lists, ix->off);
-    cudaFreeAsync(d_slot, stream);
-    cudaFreeAsync(d_flags, stream);
+    ix->built = true;
+    int rc = build_lists("siesta_index_build", L, pair_a, pair_b, n_pairs, nullptr, 0, ix->off, &ix->d_lists);
     if (rc) {
         delete ix;
         return rc;
@@ -543,4 +709,157 @@ extern "C" int siesta_intersect(siesta_index* index, const int32_t* pair_ids, in
     }
     cudaFreeAsync(d, ix->log->ctx->stream);
     return rc;
+}
+
+// ------------------------------------------------------------------------------------------------ index after a log append
+namespace {
+// the new log may carry an index of `ix`'s log: same context, no fewer traces (sets the error)
+bool index_log_ok(const char* fn, const Index* ix, const Log* L) {
+    if (L->ctx != ix->log->ctx) {
+        set_error(std::string(fn) + ": new_log is on another context than the index");
+        return false;
+    }
+    if (L->n_traces < ix->log->n_traces) {
+        set_error(std::string(fn) + ": new_log has fewer traces than the index's log");
+        return false;
+    }
+    return true;
+}
+
+// *out = a new index on L with ix's pairs and the lists d_lists / off
+int finish_index(const Index* ix, Log* L, int64_t* d_lists, std::vector<int64_t>& off, bool built, siesta_index** out) {
+    Index* nx = new Index();
+    nx->log = L;
+    nx->n_pairs = ix->n_pairs;
+    nx->pair_a = ix->pair_a;
+    nx->pair_b = ix->pair_b;
+    nx->off.swap(off);
+    nx->d_lists = d_lists;
+    nx->built = built;
+    *out = reinterpret_cast<siesta_index*>(nx);
+    return SIESTA_OK;
+}
+}  // namespace
+
+extern "C" int siesta_index_append(siesta_index* index, siesta_log* new_log, const int64_t* delta_off, const int64_t* delta_trace_idx,
+                                   siesta_index** out, double* kernel_ms) {
+    Index* ix = reinterpret_cast<Index*>(index);
+    Log* L = reinterpret_cast<Log*>(new_log);
+    if (!ix || !L || !delta_off || !out) {
+        set_error("siesta_index_append: null argument");
+        return SIESTA_E_INVALID;
+    }
+    if (!index_log_ok("siesta_index_append", ix, L)) return SIESTA_E_INVALID;
+    const int32_t n_pairs = ix->n_pairs;
+    if (delta_off[0] != 0) {
+        set_error("siesta_index_append: delta_off[0] must be 0");
+        return SIESTA_E_INVALID;
+    }
+    for (int p = 0; p < n_pairs; ++p)
+        if (delta_off[p + 1] < delta_off[p]) {
+            set_error("siesta_index_append: delta_off must be non-decreasing");
+            return SIESTA_E_INVALID;
+        }
+    const int64_t D = delta_off[n_pairs];
+    if (D > 0 && !delta_trace_idx) {
+        set_error("siesta_index_append: null delta_trace_idx");
+        return SIESTA_E_INVALID;
+    }
+    for (int p = 0; p < n_pairs; ++p)
+        for (int64_t i = delta_off[p]; i < delta_off[p + 1]; ++i)
+            if (delta_trace_idx[i] < 0 || delta_trace_idx[i] >= L->n_traces || (i > delta_off[p] && delta_trace_idx[i] <= delta_trace_idx[i - 1])) {
+                set_error("siesta_index_append: delta lists must be strictly ascending trace indices of new_log");
+                return SIESTA_E_INVALID;
+            }
+    SIESTA_CUDA_OK(cudaSetDevice(L->ctx->device));
+    cudaStream_t stream = L->ctx->stream;
+    CallScratch cs(stream);
+    int64_t* d_delta = nullptr;
+    SIESTA_CUDA_OK(cs.alloc((void**)&d_delta, sizeof(int64_t) * (size_t)std::max<int64_t>(D, 1)));
+    if (D) SIESTA_CUDA_OK(cudaMemcpyAsync(d_delta, delta_trace_idx, sizeof(int64_t) * (size_t)D, cudaMemcpyHostToDevice, stream));
+    SIESTA_CUDA_OK(cudaEventCreate(&cs.e0));
+    SIESTA_CUDA_OK(cudaEventCreate(&cs.e1));
+    SIESTA_CUDA_OK(cudaEventRecord(cs.e0, stream));
+    std::vector<int64_t> doff(delta_off, delta_off + n_pairs + 1), off;
+    int64_t* d_lists = nullptr;
+    int rc = merge_lists(stream, ix->d_lists, ix->off, d_delta, doff, n_pairs, &d_lists, off);
+    if (rc) return rc;
+    cudaError_t e = cudaEventRecord(cs.e1, stream);
+    if (e == cudaSuccess) e = cudaStreamSynchronize(stream);
+    float ms = 0.f;
+    if (e == cudaSuccess) e = cudaEventElapsedTime(&ms, cs.e0, cs.e1);
+    if (e != cudaSuccess) {
+        cudaFreeAsync(d_lists, stream);
+        set_error(std::string("siesta_index_append: ") + cudaGetErrorString(e));
+        return SIESTA_E_CUDA;
+    }
+    if (kernel_ms) *kernel_ms = ms;
+    return finish_index(ix, L, d_lists, off, false, out);
+}
+
+extern "C" int siesta_index_refresh(siesta_index* index, siesta_log* new_log, const int64_t* trace_idx, int64_t n_listed,
+                                    siesta_index** out, double* kernel_ms) {
+    Index* ix = reinterpret_cast<Index*>(index);
+    Log* L = reinterpret_cast<Log*>(new_log);
+    if (!ix || !L || !out || n_listed < 0 || (n_listed > 0 && !trace_idx)) {
+        set_error("siesta_index_refresh: null argument");
+        return SIESTA_E_INVALID;
+    }
+    if (!ix->built) {
+        set_error("siesta_index_refresh: a loaded index cannot be re-derived on the device (use siesta_index_append)");
+        return SIESTA_E_INVALID;
+    }
+    if (!index_log_ok("siesta_index_refresh", ix, L)) return SIESTA_E_INVALID;
+    const int64_t T = ix->log->n_traces, T2 = L->n_traces;
+    int64_t n_new = 0;
+    for (int64_t i = 0; i < n_listed; ++i) {
+        if (trace_idx[i] < 0 || trace_idx[i] >= T2 || (i > 0 && trace_idx[i] <= trace_idx[i - 1])) {
+            set_error("siesta_index_refresh: trace_idx must ascend strictly inside [0, new_log's n_traces)");
+            return SIESTA_E_INVALID;
+        }
+        n_new += trace_idx[i] >= T;
+    }
+    if (n_new != T2 - T) {
+        set_error("siesta_index_refresh: trace_idx must list every trace new_log adds (as passed to siesta_log_append)");
+        return SIESTA_E_INVALID;
+    }
+    // Ids outside the old log's alphabet that the new alphabet covers: when a pair names one, unlisted traces may hold it
+    // and gain the pair, so every trace is flagged again.
+    bool all = false;
+    if (!ix->log->act_valid)
+        for (int p = 0; p < ix->n_pairs; ++p)
+            for (int32_t a : {ix->pair_a[p], ix->pair_b[p]})
+                all |= a >= ix->log->n_activities && a < L->n_activities;
+    SIESTA_CUDA_OK(cudaSetDevice(L->ctx->device));
+    cudaStream_t stream = L->ctx->stream;
+    CallScratch cs(stream);
+    int64_t* d_work = nullptr;
+    if (!all) {
+        SIESTA_CUDA_OK(cs.alloc((void**)&d_work, sizeof(int64_t) * (size_t)std::max<int64_t>(n_listed, 1)));
+        if (n_listed) SIESTA_CUDA_OK(cudaMemcpyAsync(d_work, trace_idx, sizeof(int64_t) * (size_t)n_listed, cudaMemcpyHostToDevice, stream));
+    }
+    SIESTA_CUDA_OK(cudaEventCreate(&cs.e0));
+    SIESTA_CUDA_OK(cudaEventCreate(&cs.e1));
+    SIESTA_CUDA_OK(cudaEventRecord(cs.e0, stream));
+    std::vector<int64_t> doff, off;
+    int64_t *d_delta = nullptr, *d_lists = nullptr;
+    int rc = build_lists("siesta_index_refresh", L, ix->pair_a.data(), ix->pair_b.data(), ix->n_pairs, all ? nullptr : d_work, n_listed,
+                         all ? off : doff, all ? &d_lists : &d_delta);
+    if (rc) return rc;
+    if (!all) {
+        rc = merge_lists(stream, ix->d_lists, ix->off, d_delta, doff, ix->n_pairs, &d_lists, off);
+        cudaFreeAsync(d_delta, stream);
+        if (rc) return rc;
+    }
+    cudaError_t e = cudaEventRecord(cs.e1, stream);
+    if (e == cudaSuccess) e = cudaStreamSynchronize(stream);
+    float ms = 0.f;
+    if (e == cudaSuccess) e = cudaEventElapsedTime(&ms, cs.e0, cs.e1);
+    if (e != cudaSuccess) {
+        cudaFreeAsync(d_lists, stream);
+        set_error(std::string("siesta_index_refresh: ") + cudaGetErrorString(e));
+        return SIESTA_E_CUDA;
+    }
+    if (kernel_ms) *kernel_ms = ms;
+    return finish_index(ix, L, d_lists, off, true, out);
 }
