@@ -658,6 +658,10 @@ struct GatherParams {
     int32_t* ev_act;
     int64_t* ev_ts;
     int all_cols;
+    // uniform placement: K1-P's tile words ([2][n_tiles], DetectParams::tile_words) and its fixed staging slots
+    const uint32_t* tile_words;
+    int64_t n_tiles;
+    int64_t fix_ev;
 };
 
 template <int NTHR = GT>
@@ -823,65 +827,169 @@ __global__ void __launch_bounds__(GT) gather_kernel(const __grid_constant__ Gath
     }
 }
 
-// The same placement when every matching trace holds ONE occurrence of k events (class NK asked for the first-largest
-// occurrence: the metric's configuration).  The three running sums collapse into one count of matching traces - a ballot and
-// a popcount per warp instead of three 64-bit shuffle scans - and the owner of an output slot is found through a
-// 32-entry table in shared memory instead of a five-step shuffle search: the general kernel spends ~470 instructions per
-// candidate (profiles/r02c_gather_ncu_summary.md), this one a third of that.
-__global__ void __launch_bounds__(GT) gather_uniform_kernel(const __grid_constant__ GatherParams G, const int k) {
-    __shared__ unsigned s_wsum[GT / 32];
-    __shared__ long long s_se[GT / 32][32];
-    const int64_t i = (int64_t)blockIdx.x * GT + threadIdx.x;
+// The compact block of the multi-GPU exchange (layout: pack_layout below).
+struct PackSections {
+    uint32_t* trace;
+    int64_t* base;
+    uint32_t *occ_off, *ev_off;
+    uint16_t* pos;
+    uint8_t* rank;
+    uint16_t* act;
+    int32_t* delta;
+    int64_t* err;
+    int64_t* unsup;
+    int32_t seconds;
+    int* status;
+};
+
+// The placement when every matching trace holds ONE occurrence of k events (class NK asked for the first-largest
+// occurrence: the metric's configuration), into the result columns (PACK = false) or into the exchange's compact block
+// (PACK = true).  One warp per block of 256 candidates, the granularity of the block sums, so its first row is known
+// from the scanned sums alone.
+//   rows     K1-P left two words per tile of 32 candidates (DetectParams::tile_words): the lanes that matched and the
+//            lanes it sent to the overflow list.  Only the overflow lanes read d_cnt / d_stage, which the staged
+//            kernels and K1-L wrote for exactly those candidates; a lane's row is the popcount of the matching lanes
+//            below it.  Without K1-P every lane is marked overflow, so every candidate is read as the staged kernel left it.
+//   events   a K1-P match's k events sit at its tile's fixed slots in lane order, one word {pos, rank, act} and the
+//            timestamp each; a re-run trace's at d_stage in the four staged columns.  Where every row of a block comes
+//            from K1-P the block's events are 8 contiguous runs; they are copied 128 per step, all loads of a step
+//            issued before its first store.
+template <bool PACK>
+__global__ void __launch_bounds__(GT) gather_uniform_kernel(const __grid_constant__ GatherParams G, const __grid_constant__ PackSections O,
+                                                            const int k) {
+    __shared__ long long s_src[GT / 32][256];   // per row of the block: K1-P slot (>= 0) or ~d_stage of a re-run trace
     const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
-    const int64_t chunk = blockIdx.x / SC;
-    const unsigned long long b0 = G.top[chunk] + G.blk[blockIdx.x];   // matching traces before this block (sum 0 of 3)
+    const int64_t blk = (int64_t)blockIdx.x * (GT / 32) + warp;
+    if (blk >= G.n_blk) return;
+    long long* src = s_src[warp];
+    const uint32_t below = (1u << lane) - 1u;
+    const int64_t t0 = blk * 8;
+    // the tile words: lanes 0-7 the matched lanes of the block's tiles, lanes 8-15 the overflow lanes
     uint32_t w = 0;
-    long long se = 0;
-    int64_t cand_i = i;
-    if (i < G.n) {
-        w = G.d_cnt[i];
-        se = G.d_stage[i];
-        if (G.cand) cand_i = G.cand[i];
-    }
-    const bool hit = (w & 0xFFFFu) != 0;
-    const unsigned bal = __ballot_sync(0xffffffffu, hit);
-    const unsigned wex = __popc(bal & ((1u << lane) - 1u));
-    const unsigned wn = __popc(bal);
-    if (lane == 0) s_wsum[warp] = wn;
-    if (hit) s_se[warp][wex] = se;   // the r-th matching trace of the warp: where its k events are staged
-    __syncthreads();
-    unsigned before = 0;
+    if (lane < 16 && t0 + (lane & 7) < G.n_tiles) w = __ldg(G.tile_words + (lane < 8 ? 0 : G.n_tiles) + t0 + (lane & 7));
+    const unsigned long long b0 = G.top[blk / SC] + G.blk[blk];   // matching traces before this block (sum 0 of 3)
+    uint32_t mw[8], full[8];
+    long long se[8];
+    uint32_t any_ovf = 0;
 #pragma unroll
-    for (int q = 0; q < GT / 32; ++q) before += q < warp ? s_wsum[q] : 0u;
-    const int64_t wtp = (int64_t)b0 + before;   // matching traces before this warp
-    if (hit) {
-        const int64_t tp = wtp + wex;
-        G.trace_idx[tp] = cand_i + G.base.trace;
-        G.occ_off[tp] = tp + G.base.occ;
-        G.ev_off[tp] = tp * k + G.base.ev;
+    for (int j = 0; j < 8; ++j) {
+        mw[j] = __shfl_sync(0xffffffffu, w, j);
+        full[j] = __shfl_sync(0xffffffffu, w, 8 + j);   // (overflow lanes for now)
+        any_ovf |= full[j];
+        se[j] = 0;
     }
-    const unsigned wtot = wn * (unsigned)k;
-    const long long wbase = wtp * k;
+    if (any_ovf) {   // re-run traces in the block (uniform branch)
+        uint32_t cnt[8];
+#pragma unroll
+        for (int j = 0; j < 8; ++j) {
+            const int64_t c = blk * 256 + j * 32 + lane;
+            cnt[j] = 0;
+            if (((full[j] >> lane) & 1u) && c < G.n) {
+                cnt[j] = G.d_cnt[c];
+                se[j] = G.d_stage[c];
+            }
+        }
+#pragma unroll
+        for (int j = 0; j < 8; ++j) full[j] = mw[j] | __ballot_sync(0xffffffffu, (cnt[j] & 0xFFFFu) != 0);
+    } else {
+#pragma unroll
+        for (int j = 0; j < 8; ++j) full[j] = mw[j];
+    }
+    // rows: the trace columns, and where each row's events are staged
+    unsigned n_rows = 0;
+    int bad = 0;
+    int64_t cid[8];
+#pragma unroll
+    for (int j = 0; j < 8; ++j) {
+        const int64_t c = blk * 256 + j * 32 + lane;
+        cid[j] = (!PACK && G.cand && ((full[j] >> lane) & 1u)) ? __ldg(G.cand + c) : c;
+    }
+#pragma unroll
+    for (int j = 0; j < 8; ++j) {
+        if ((full[j] >> lane) & 1u) {
+            const unsigned r = n_rows + __popc(full[j] & below);
+            src[r] = ((mw[j] >> lane) & 1u) ? G.fix_ev + (t0 + j) * 32 * k + (long long)__popc(mw[j] & below) * k : ~se[j];
+            const int64_t tp = (int64_t)b0 + r;
+            if constexpr (PACK) {
+                bad |= (unsigned long long)cid[j] > 0xFFFFFFFFull;
+                O.trace[tp] = (uint32_t)cid[j];   // no candidate list on the exchange path: the shard-local trace index
+            } else {
+                G.trace_idx[tp] = cid[j] + G.base.trace;
+                G.occ_off[tp] = tp + G.base.occ;
+                G.ev_off[tp] = tp * k + G.base.ev;
+            }
+        }
+        n_rows += __popc(full[j]);
+    }
+    __syncwarp();
+    const unsigned tot = n_rows * (unsigned)k;   // <= 2048
+    const long long ebase = (long long)b0 * k;
     const unsigned inv = 65536u / (unsigned)k + 1u;   // (f * inv) >> 16 == f / k for every f < 2048 and k <= 8
-    for (unsigned f = lane; f < wtot; f += 32) {
-        const unsigned r = (f * inv) >> 16, e = f - r * (unsigned)k;
-        const long long from = s_se[warp][r] + e;
-        const long long to = wbase + f;
-        const int32_t c_pos = __ldg(G.s_ev_pos + from);
-        int32_t c_rank = 0, c_act = 0;
-        long long c_ts = 0;
-        if (G.all_cols) {
-            c_rank = __ldg(G.s_ev_rank + from);
-            c_act = __ldg(G.s_ev_act + from);
-            c_ts = __ldg(reinterpret_cast<const long long*>(G.s_ev_ts) + from);
+    const long long* s_ts = reinterpret_cast<const long long*>(G.s_ev_ts);
+    for (unsigned f0 = 0; f0 < tot; f0 += 128) {
+        int32_t v_pos[4], v_rank[4], v_act[4];
+        long long v_ts[4], v_t0[4];
+        bool packed[4];
+#pragma unroll
+        for (int u = 0; u < 4; ++u) {
+            const unsigned f = f0 + 32 * u + lane;
+            v_pos[u] = v_rank[u] = v_act[u] = 0;
+            v_ts[u] = v_t0[u] = 0;
+            packed[u] = true;
+            if (f < tot) {
+                const unsigned r = (f * inv) >> 16, e = f - r * (unsigned)k;
+                long long s = src[r];
+                packed[u] = s >= 0;
+                if (!packed[u]) s = ~s;
+                v_pos[u] = __ldg(G.s_ev_pos + s + e);
+                if (G.all_cols) {
+                    if (!packed[u]) {
+                        v_rank[u] = __ldg(G.s_ev_rank + s + e);
+                        v_act[u] = __ldg(G.s_ev_act + s + e);
+                    }
+                    v_ts[u] = __ldg(s_ts + s + e);
+                    if (PACK) v_t0[u] = __ldg(s_ts + s);   // the row's first event: base of the deltas
+                }
+            }
         }
-        G.ev_posv[to] = c_pos;
-        if (G.all_cols) {
-            G.ev_rank[to] = c_rank;
-            G.ev_act[to] = c_act;
-            G.ev_ts[to] = c_ts;
+#pragma unroll
+        for (int u = 0; u < 4; ++u) {
+            const unsigned f = f0 + 32 * u + lane;
+            if (f >= tot) continue;
+            if (packed[u]) {
+                const uint32_t x = (uint32_t)v_pos[u];
+                v_pos[u] = (int32_t)(x & 0xFFu);
+                v_rank[u] = (int32_t)((x >> 8) & 0xFFu);
+                v_act[u] = (int32_t)(x >> 16);
+            }
+            const long long to = ebase + f;
+            if constexpr (PACK) {
+                bad |= (unsigned)v_pos[u] > 0xFFFFu;
+                O.pos[to] = (uint16_t)v_pos[u];
+                if (G.all_cols) {
+                    const unsigned r = (f * inv) >> 16;
+                    if (f == r * (unsigned)k) O.base[(int64_t)b0 + r] = v_ts[u];
+                    long long d = v_ts[u] - v_t0[u];
+                    if (O.seconds) {
+                        bad |= d % 1000 != 0;
+                        d /= 1000;
+                    }
+                    bad |= (unsigned)v_rank[u] > 0xFFu || (unsigned)v_act[u] > 0xFFFFu || d < -0x7fffffffll - 1 || d > 0x7fffffffll;
+                    O.rank[to] = (uint8_t)v_rank[u];
+                    O.act[to] = (uint16_t)v_act[u];
+                    O.delta[to] = (int32_t)d;
+                }
+            } else {
+                G.ev_posv[to] = v_pos[u];
+                if (G.all_cols) {
+                    G.ev_rank[to] = v_rank[u];
+                    G.ev_act[to] = v_act[u];
+                    G.ev_ts[to] = v_ts[u];
+                }
+            }
         }
     }
+    if (PACK && __any_sync(0xffffffffu, bad) && lane == 0) atomicOr(O.status, XST_RANGE);
 }
 
 __global__ void set_tail_kernel(int64_t* occ_off, int64_t n_tr, int64_t n_occ, int64_t* ev_off, int64_t n_ev, RebaseOffsets base) {
@@ -972,6 +1080,8 @@ struct DetectPending {
     int unsup_slot = 7;                   // counter that counts them (7: wide launch, 14: K1-L)
     void* work = nullptr;                 // scratch of the call (freed by the second half)
     int uniform_k = 0;                    // > 0: one occurrence per trace, uniform_k events each (class NK, first-largest)
+    const uint32_t* tile_words = nullptr; // set: the uniform placement (gather_uniform_kernel) places the result
+    int64_t n_tiles = 0, fix_ev = 0;
     cudaEvent_t ev0 = nullptr, evd = nullptr;
     unsigned long long* h_cnt = nullptr;  // pinned, 16 words
     const uint16_t* d_lut = nullptr;      // the request's tables on the device (a later block of the same request reuses them)
@@ -1032,7 +1142,8 @@ int detect_device_begin_impl(Log* log, const siesta_nfa* nfa, const int64_t* d_c
     // trace's filtered events (<= 64 on the widest engine configuration)
     const int64_t wide = std::min<int64_t>(log->n_events, n * 64);
     const int64_t cap_occ = return_all ? wide : n;
-    const int64_t cap_ev = (!return_all && !dn.any_kleene) ? n * std::max(1, n_positive) : wide;
+    const int uniform_k = (!return_all && !dn.any_kleene) ? std::max(1, n_positive) : 0;
+    const int64_t cap_ev = uniform_k ? n * uniform_k : wide;
 
     // one stream-ordered allocation for all scratch of the call, carved by a bump pointer
     DevBuf work(log->ctx);
@@ -1069,6 +1180,10 @@ int detect_device_begin_impl(Log* log, const siesta_nfa* nfa, const int64_t* d_c
     const int64_t cap_long = use_long ? std::min<int64_t>(log->n_events, (int64_t)1 << 21) : 0;
     const size_t long_pool = use_long ? (size_t)std::min<int64_t>(std::max<int64_t>(log->n_events * 64, (int64_t)1 << 20), (int64_t)256 << 20) : 0;
     const size_t n_blk = (nn + GT - 1) / GT;
+    // a uniform result is placed by gather_uniform_kernel from two words per tile of 32 candidates
+    const bool uniform_place = uniform_k > 0 && uniform_k <= 8 && std::getenv("SIESTA_NO_UNIFORM_GATHER") == nullptr;
+    const size_t n_tiles = (nn + 31) / 32;
+    const size_t o_tiles = uniform_place ? carve(n_tiles * 2 * 4) : 0;
     const size_t o_ovf2 = use_nkp ? carve(nn * 8) : 0;
     const size_t o_unsup = carve((size_t)SIESTA_MAX_UNSUPPORTED * 8);   // traces beyond the engine limits (wide launch)
     const size_t o_unsup2 = use_long ? carve((size_t)SIESTA_MAX_UNSUPPORTED * 8) : 0;   // ... and beyond K1-L's pool / staging
@@ -1173,9 +1288,15 @@ int detect_device_begin_impl(Log* log, const siesta_nfa* nfa, const int64_t* d_c
         return SIESTA_E_NOMEM;
     }
     std::memset(h_cnt, 0, 128);
+    uint32_t* tile_words = uniform_place ? reinterpret_cast<uint32_t*>(wb + o_tiles) : nullptr;
     if (n > 0) {
+        if (uniform_place && !use_nkp) {   // no K1-P: every lane is an overflow lane, its d_cnt is read
+            SIESTA_CUDA_OK(cudaMemsetAsync(tile_words, 0, n_tiles * 4, stream));
+            SIESTA_CUDA_OK(cudaMemsetAsync(tile_words + n_tiles, 0xFF, n_tiles * 4, stream));
+        }
         if (use_nkp) {
             DetectParams N = P;
+            N.tile_words = tile_words;
             N.ovf_list = reinterpret_cast<int64_t*>(wb + o_ovf2);
             N.ovf_slot = 13;
             N.tile_slot = 18;
@@ -1280,7 +1401,10 @@ int detect_device_begin_impl(Log* log, const siesta_nfa* nfa, const int64_t* d_c
     q->d_unsup = reinterpret_cast<int64_t*>(wb + (use_long ? o_unsup2 : o_unsup));
     q->unsup_slot = use_long ? 14 : 7;
     q->work = work.release();
-    q->uniform_k = (!return_all && !dn.any_kleene) ? std::max(1, n_positive) : 0;
+    q->uniform_k = uniform_k;
+    q->tile_words = tile_words;
+    q->n_tiles = (int64_t)n_tiles;
+    q->fix_ev = cap_ev;
     q->ev0 = ev0;
     q->evd = evd;
     q->h_cnt = h_cnt;
@@ -1386,14 +1510,19 @@ int detect_device_finish_impl(DetectPending* q, siesta_dev_matches* out) {
         G.ev_act = f_act.as<int32_t>();
         G.ev_ts = f_ts.as<int64_t>();
         G.all_cols = all_cols ? 1 : 0;
+        G.tile_words = q->tile_words;
+        G.n_tiles = q->n_tiles;
+        G.fix_ev = q->fix_ev;
         // (the block sums were accumulated by the verification kernels: no counting pass)
         scan_chunks_kernel<<<(unsigned)G.n_chunks, SC, 0, stream>>>(G.blk, G.n_blk, G.top, G.n_chunks);
         SIESTA_LAUNCHED();
         scan_top_kernel<<<1, SC, 0, stream>>>(G.top, G.n_chunks);
         SIESTA_LAUNCHED();
-        if (q->uniform_k > 0 && q->uniform_k <= 8 && std::getenv("SIESTA_NO_UNIFORM_GATHER") == nullptr)
-            gather_uniform_kernel<<<(unsigned)G.n_blk, GT, 0, stream>>>(G, q->uniform_k);
-        else
+        if (q->tile_words) {
+            PackSections none;
+            std::memset(&none, 0, sizeof(none));
+            gather_uniform_kernel<false><<<(unsigned)((G.n_blk + GT / 32 - 1) / (GT / 32)), GT, 0, stream>>>(G, none, q->uniform_k);
+        } else
             gather_kernel<<<(unsigned)G.n_blk, GT, 0, stream>>>(G);
         SIESTA_LAUNCHED();
         SIESTA_CUDA_OK(cudaGetLastError());
@@ -1466,19 +1595,6 @@ int detect_device_finish_impl(DetectPending* q, siesta_dev_matches* out) {
 //   pos u16[n_ev]  rank u8[n_ev]  act u16[n_ev]  delta i32[n_ev]  (ev_ts_ms - base) in seconds (EventTs route: exact,
 //                                                           both are rel_s * 1000 + t0) or milliseconds (EventPos route)
 //   err      i64[n_err] shard-local indices of the traces on which the Java engine would throw (<= XCHG_ERR_CAP)
-struct PackSections {
-    uint32_t* trace;
-    int64_t* base;
-    uint32_t *occ_off, *ev_off;
-    uint16_t* pos;
-    uint8_t* rank;
-    uint16_t* act;
-    int32_t* delta;
-    int64_t* err;
-    int64_t* unsup;
-    int32_t seconds;
-    int* status;
-};
 static inline size_t al256(size_t x) { return (x + 255) & ~(size_t)255; }
 // byte offsets of the sections inside the data area, from the capacities; returns the bytes needed
 static size_t pack_layout(int64_t n, int64_t cap_occ, int64_t cap_ev, int uniform_k, bool all_cols, XHeader* h) {
@@ -1587,74 +1703,6 @@ __global__ void __launch_bounds__(GT) gather_packed_kernel(const __grid_constant
                 O.act[to] = (uint16_t)c_act;
                 O.delta[to] = (int32_t)d;
             }
-        }
-    }
-    if (__any_sync(0xffffffffu, bad) && lane == 0) atomicOr(O.status, XST_RANGE);
-}
-
-// The compact block when every matching trace holds one occurrence of k events (gather_uniform_kernel's counting, the
-// wire format of gather_packed_kernel with uniform = 1: no offset sections).
-__global__ void __launch_bounds__(GT) gather_packed_uniform_kernel(const __grid_constant__ GatherParams G, const __grid_constant__ PackSections O,
-                                                                   const int k) {
-    __shared__ unsigned s_wsum[GT / 32];
-    __shared__ long long s_se[GT / 32][32];
-    const int64_t i = (int64_t)blockIdx.x * GT + threadIdx.x;
-    const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
-    const int64_t chunk = blockIdx.x / SC;
-    const unsigned long long b0 = G.top[chunk] + G.blk[blockIdx.x];
-    uint32_t w = 0;
-    long long se = 0;
-    if (i < G.n) {
-        w = G.d_cnt[i];
-        se = G.d_stage[i];
-    }
-    const bool hit = (w & 0xFFFFu) != 0;
-    const unsigned bal = __ballot_sync(0xffffffffu, hit);
-    const unsigned wex = __popc(bal & ((1u << lane) - 1u));
-    const unsigned wn = __popc(bal);
-    if (lane == 0) s_wsum[warp] = wn;
-    if (hit) s_se[warp][wex] = se;
-    __syncthreads();
-    unsigned before = 0;
-#pragma unroll
-    for (int q = 0; q < GT / 32; ++q) before += q < warp ? s_wsum[q] : 0u;
-    const int64_t wtp = (int64_t)b0 + before;
-    int bad = 0;
-    if (hit) {
-        const int64_t tp = wtp + wex;
-        bad |= (unsigned long long)i > 0xFFFFFFFFull;
-        O.trace[tp] = (uint32_t)i;
-        if (O.base) O.base[tp] = G.s_ev_ts[se];
-    }
-    const unsigned wtot = wn * (unsigned)k;
-    const long long wbase = wtp * k;
-    const unsigned inv = 65536u / (unsigned)k + 1u;   // (f * inv) >> 16 == f / k for every f < 2048 and k <= 8
-    for (unsigned f = lane; f < wtot; f += 32) {
-        const unsigned r = (f * inv) >> 16, e = f - r * (unsigned)k;
-        const long long o_se = s_se[warp][r];
-        const long long from = o_se + e;
-        const long long to = wbase + f;
-        const int32_t c_pos = __ldg(G.s_ev_pos + from);
-        int32_t c_rank = 0, c_act = 0;
-        long long c_ts = 0, c_base = 0;
-        if (G.all_cols) {
-            c_rank = __ldg(G.s_ev_rank + from);
-            c_act = __ldg(G.s_ev_act + from);
-            c_ts = __ldg(reinterpret_cast<const long long*>(G.s_ev_ts) + from);
-            c_base = __ldg(reinterpret_cast<const long long*>(G.s_ev_ts) + o_se);
-        }
-        bad |= (unsigned)c_pos > 0xFFFFu;
-        O.pos[to] = (uint16_t)c_pos;
-        if (G.all_cols) {
-            long long d = c_ts - c_base;
-            if (O.seconds) {
-                bad |= d % 1000 != 0;
-                d /= 1000;
-            }
-            bad |= (unsigned)c_rank > 0xFFu || (unsigned)c_act > 0xFFFFu || d < -0x7fffffffll - 1 || d > 0x7fffffffll;
-            O.rank[to] = (uint8_t)c_rank;
-            O.act[to] = (uint16_t)c_act;
-            O.delta[to] = (int32_t)d;
         }
     }
     if (__any_sync(0xffffffffu, bad) && lane == 0) atomicOr(O.status, XST_RANGE);
@@ -1799,12 +1847,15 @@ int detect_device_pack_impl(DetectPending* q, const PackTarget& tgt) {
         G.s_ev_act = P.s_ev_act;
         G.s_ev_ts = P.s_ev_ts;
         G.all_cols = all_cols ? 1 : 0;
+        G.tile_words = q->tile_words;
+        G.n_tiles = q->n_tiles;
+        G.fix_ev = q->fix_ev;
         scan_chunks_kernel<<<(unsigned)G.n_chunks, SC, 0, stream>>>(G.blk, G.n_blk, G.top, G.n_chunks);
         SIESTA_LAUNCHED();
         scan_top_kernel<<<1, SC, 0, stream>>>(G.top, G.n_chunks);
         SIESTA_LAUNCHED();
-        if (q->uniform_k > 0 && q->uniform_k <= 8 && std::getenv("SIESTA_NO_UNIFORM_GATHER") == nullptr)
-            gather_packed_uniform_kernel<<<(unsigned)G.n_blk, GT, 0, stream>>>(G, O, q->uniform_k);
+        if (q->tile_words)
+            gather_uniform_kernel<true><<<(unsigned)((G.n_blk + GT / 32 - 1) / (GT / 32)), GT, 0, stream>>>(G, O, q->uniform_k);
         else
             gather_packed_kernel<<<(unsigned)G.n_blk, GT, 0, stream>>>(G, O, q->uniform_k ? 1 : 0);
         SIESTA_LAUNCHED();

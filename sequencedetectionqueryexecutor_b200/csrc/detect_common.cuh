@@ -52,6 +52,11 @@ struct DetectParams {
     int64_t fix_ev;
     int32_t fix_np;
     int64_t fix_occ;          // returnAll: candidate i stages its occurrence's event count at s_occ_nev[fix_occ + i] (-1: not asked for)
+    // K1-P, uniform result (one occurrence of fix_np events per matching trace): per tile the lanes that matched
+    // (tile_words[tile]) and the lanes sent to the overflow list (tile_words[n_tiles + tile]); each event is staged as
+    // one word pos | rank << 8 | act << 16 in s_ev_pos plus its timestamp, and no d_cnt / d_stage is written for the
+    // traces K1-P answers.  nullptr: the per-candidate outputs and the four staged columns
+    uint32_t* tile_words;
     // K1-P: a state that owns exactly ONE class is the minterm of the class planes with these polarities
     // (st_inv[k][p] = 0 or ~0: plane p enters state k's mask as it is / complemented); st_single[k] = 0: OR of several classes
     uint32_t st_inv[SIESTA_MAX_STATES][3];

@@ -21,7 +21,9 @@
 //   walk     NkwWalk: per state one AND of {state mask, above(previous event), predicate windows} and a lowest-set-bit;
 //            the first start whose walk completes is the first-largest occurrence (monotone walks)
 //   output   fixed staging slots per tile (no atomic on the critical path), the tile's events written as one flat
-//            coalesced stream; the placement kernels of detect.cu order them by trace
+//            coalesced stream; the placement kernels of detect.cu order them by trace.  A uniform result is staged for
+//            gather_uniform_kernel: two words per tile (matched / overflow lanes) instead of per-candidate counts, one
+//            packed {pos, rank, act} word and the timestamp per event
 // Traces that do not fit (more than 64 slots, or more than 32 relevant events in rank space) go to the overflow list
 // and re-run on the staged kernel, launched unconditionally with its work count read from the device.
 #include "detect_common.cuh"
@@ -244,7 +246,8 @@ __global__ void __launch_bounds__(NT_MAX, SIESTA_NKP_MIN_CTAS) detect_nkp_kernel
                 if (lane >= d) i2 += y2;
             }
         }
-        const unsigned n_match = __popc(__ballot_sync(0xffffffffu, status == ST_MATCH));
+        const unsigned match_bal = __ballot_sync(0xffffffffu, status == ST_MATCH);
+        const unsigned n_match = __popc(match_bal);
         acc_occ += n_match;
         acc_ev += i1;     // lane 31 holds the tile totals
         acc_emit += i2;
@@ -256,7 +259,16 @@ __global__ void __launch_bounds__(NT_MAX, SIESTA_NKP_MIN_CTAS) detect_nkp_kernel
             atomicAdd(b + 2 * P.n_blk, (unsigned long long)i1);
         }
         const long long base1 = P.fix_ev + tile * 32 * P.fix_np;
-        if (ci >= 0) {
+        const bool uniform = P.tile_words != nullptr;
+        if (uniform) {   // the tile's two words replace the per-candidate count and staging place
+            const unsigned ovf_bal = __ballot_sync(0xffffffffu, status == ST_OVF);
+            if (lane == 0) P.tile_words[tile] = match_bal;
+            if (lane == 1) P.tile_words[n_tiles + tile] = ovf_bal;
+            if (status == ST_OVF) {
+                const unsigned long long at = atomicAdd(P.counters + P.ovf_slot, 1ull);
+                P.ovf_list[at] = ci;
+            }
+        } else if (ci >= 0) {
             P.d_cnt[ci] = my_occ | (my_ev << 16);
             if (status == ST_MATCH) {
                 P.d_stage[ci] = base1 + (long long)(i1 - my_ev);
@@ -300,16 +312,21 @@ __global__ void __launch_bounds__(NT_MAX, SIESTA_NKP_MIN_CTAS) detect_nkp_kernel
                     }
                     const int src = j - (int)(o_o0 & 7);
                     const long long at = base1 + f;
-                    P.s_ev_pos[at] = src;
-                    if (all_cols) {
+                    if (!all_cols) P.s_ev_pos[at] = src;
+                    else {
                         // all three loads leave together: the event's activity and timestamp, and the timestamp of the
                         // first event of the filtered list (Utils.java:51-53: base of the EventTs route's seconds)
                         const long long* tsp = reinterpret_cast<const long long*>(P.ts_ms) + o_o0;
                         const int32_t c_act = __ldg(P.act + o_o0 + src);
                         const long long raw = __ldg(tsp + src);
                         const long long o_t0 = evt_pos ? 0 : __ldg(tsp + (__ffsll((long long)o_R) - 1 - (int)(o_o0 & 7)));
-                        P.s_ev_rank[at] = rank;
-                        P.s_ev_act[at] = c_act;
+                        if (uniform) {   // src, rank < 64 and act < 255 (at most 64 slots, at most 255 activities)
+                            P.s_ev_pos[at] = src | (rank << 8) | (c_act << 16);
+                        } else {
+                            P.s_ev_pos[at] = src;
+                            P.s_ev_rank[at] = rank;
+                            P.s_ev_act[at] = c_act;
+                        }
                         // SaseEvent.getEventBoth: timestamp * 1000 + minTs (SaseEvent.java:94-106)
                         P.s_ev_ts[at] = evt_pos ? raw : (long long)rel_seconds(raw - o_t0) * 1000 + o_t0;
                     }
