@@ -433,6 +433,13 @@ int siesta_multi_log_append(siesta_multi_log* log, const int64_t* trace_idx, con
 int siesta_multi_detect(siesta_multi_log* log, const siesta_nfa* nfa, uint32_t flags, siesta_matches** out);
 /* = siesta_declare_counts(whole log): kernel K3 per shard + one sum all-reduce over the exchange. */
 int siesta_multi_declare_counts(siesta_multi_log* log, int32_t k_cap, int64_t* out, double* kernel_ms);
+/* = siesta_declare_counts_refresh over all shards (new_log = siesta_multi_log_append(old_log, ...)): trace_idx are GLOBAL
+ * and split as the append splits them (new traces on the last shard).  Every shard is checked before anything is
+ * counted; each computes its delta, one sum all-reduce joins them and one merge adds them to old_counts.  The count array
+ * must fit the exchange region, as for siesta_multi_declare_counts.  Same refusals and fallback. */
+int siesta_multi_declare_counts_refresh(siesta_multi_log* old_log, siesta_multi_log* new_log, const int64_t* trace_idx,
+                                        int64_t n_listed, int32_t k_cap, const int64_t* old_counts, int64_t* out,
+                                        double* kernel_ms);
 /* siesta_why_not_match (below) over all shards: cand = ascending GLOBAL trace indices (NULL: every trace); every
  * device answers its own candidates, the answers are concatenated in trace order. */
 struct siesta_wnm_constraint;
@@ -526,6 +533,34 @@ int64_t siesta_declare_counts_size(int32_t n_activities, int32_t k_cap);
 int siesta_declare_counts(siesta_log* log, int32_t k_cap, int64_t* out /* host, _size() values */, double* kernel_ms);
 int siesta_declare_counts_device(siesta_log* log, int32_t k_cap, int64_t* d_out /* device */, void* stream,
                                  double* kernel_ms);
+/* After siesta_log_append: the counts of new_log from those of old_log, recounting only the traces the batch listed.
+ * Every block of the packed result is a sum of per-trace contributions and an append changes only the listed traces, so
+ *     counts(new_log) = counts(old_log) - K3(old_log, listed old traces) + K3(new_log, listed traces)
+ * in wrapping int64 arithmetic, with old_counts moved to new_log's alphabet (new rows and columns zero).  The result
+ * equals siesta_declare_counts(new_log, k_cap) bit for bit.  Cost: 4 B per event of the listed traces in both logs,
+ * 8 B per listed trace, one read and one write of the count array, 16 B per old trace for the check below.
+ *   old_counts: siesta_declare_counts(old_log, k_cap) with the same k_cap, or an earlier refresh; laid out for old_log's
+ *               alphabet (siesta_declare_counts_size(old A, k_cap) values).  out: laid out for new_log's alphabet.
+ *   trace_idx:  exactly what siesta_log_append was given (strictly ascending, listing every new trace); across chained
+ *               appends, the union of the batches' lists.  NULL when n_listed == 0.
+ * old_log is only read and must stay alive during the call.  *kernel_ms (may be NULL) = device time between CUDA events on
+ * the call's stream, from after the host -> device copy of trace_idx to the end of the merge (the check included).
+ * One fallback: when old_log holds activity ids outside its alphabet (not every id lies in [0, n_activities)) and new_log's
+ * alphabet is larger, unlisted traces may gain counted events, so the call counts new_log in full (still exact).
+ * SIESTA_E_INVALID (nothing kept allocated, out untouched): a null argument, k_cap < 1, logs on different contexts, a
+ * derived (siesta_log_filter_time / siesta_log_group) or block-cyclic log, new_log with fewer traces or a smaller alphabet
+ * than old_log, trace_idx not strictly ascending inside [0, new_log's n_traces) or not listing every new trace, and an
+ * unlisted trace whose length differs between the two logs (one device pass over both offset arrays).
+ * SIESTA_E_UNSUPPORTED: new_log's alphabet above 4096, as siesta_declare_counts.
+ * _device: d_old / d_out are device arrays; d_out may be d_old only when the alphabet did not grow.
+ * Measured on one B200 at 1000 W (100 M traces x 50 events, 1 M touched traces x 5 events + 1 M new traces x 50 events):
+ * 3.6 / 54 / 117 ms at 20 / 100 / 400 activities against 96 / 1 733 / 4 203 ms for siesta_declare_counts on the new log.
+ * A batch that touches most traces is cheaper to count in full (both versions of every listed trace are counted). */
+int siesta_declare_counts_refresh(siesta_log* old_log, siesta_log* new_log, const int64_t* trace_idx, int64_t n_listed,
+                                  int32_t k_cap, const int64_t* old_counts /* host */, int64_t* out /* host */,
+                                  double* kernel_ms);
+int siesta_declare_counts_refresh_device(siesta_log* old_log, siesta_log* new_log, const int64_t* trace_idx, int64_t n_listed,
+                                         int32_t k_cap, const int64_t* d_old, int64_t* d_out, void* stream, double* kernel_ms);
 
 /* ------------------------------------------------------------- pair statistics */
 /* Kernel K4.  The record /stats returns per consecutive pair of the pattern (QueryPlanStats.execute, model/Queries/

@@ -30,6 +30,10 @@ final class GpuNative {
     static native int[] matchesInts(long matches, int which);     // 0 ev_pos, 1 ev_rank, 2 ev_act
     static native void matchesFree(long matches);
     static native long[] declareCounts(long log, int nActivities, int kCap);
+    // the counts of newLog (grown from oldLog by logAppend) from oldLog's, recounting only the traces traceIdx lists
+    // (global, ascending; the union over chained appends); oldCounts holds the counts of oldNActivities activities
+    static native long[] declareCountsRefresh(long oldLog, long newLog, long[] traceIdx, long[] oldCounts, int oldNActivities,
+                                              int nActivities, int kCap);
     // why-not-match (WhyNotMatchSASE.evaluate): constraints = 5 longs each (posA, posB, kind 0 gap | 1 time, method 0 within | 1 atleast, value)
     static native long whyNotMatch(long log, int[] pattern, long[] constraints, int uncertainty, int step, int k, long[] cand, int flags);
     static native long[] almostLongs(long almost, int which);    // 0 trace_idx, 1 unsupported_trace_idx

@@ -277,6 +277,43 @@ NATIVE(jlongArray, declareCounts)(JNIEnv* env, jclass cls, jlong log, jint nActi
     return out;
 }
 
+/* long[] declareCountsRefresh(long oldLog, long newLog, long[] traceIdx, long[] oldCounts, int oldNActivities, int nActivities,
+ * int kCap): the counts of newLog (= logAppend(oldLog, ...), or a chain of appends) from those of oldLog, recounting only
+ * the listed traces (traceIdx: global, ascending, the union of the appends' lists); equals declareCounts(newLog, ...)
+ * (siesta_multi_declare_counts_refresh).  oldCounts must be laid out for oldNActivities. */
+NATIVE(jlongArray, declareCountsRefresh)(JNIEnv* env, jclass cls, jlong oldLog, jlong newLog, jlongArray traceIdx, jlongArray oldCounts,
+                                         jint oldNActivities, jint nActivities, jint kCap) {
+    (void)cls;
+    const int64_t n_old = siesta_declare_counts_size((int32_t)oldNActivities, (int32_t)kCap);
+    const int64_t n = siesta_declare_counts_size((int32_t)nActivities, (int32_t)kCap);
+    if ((int64_t)(*env)->GetArrayLength(env, oldCounts) != n_old) {
+        throw_class(env, "java/lang/IllegalArgumentException", "declareCountsRefresh: oldCounts does not hold the counts of oldNActivities activities");
+        return NULL;
+    }
+    const jsize nl = (*env)->GetArrayLength(env, traceIdx);
+    int64_t* idx = (int64_t*)malloc(sizeof(int64_t) * (size_t)(nl ? nl : 1));
+    int64_t* old = (int64_t*)malloc(sizeof(int64_t) * (size_t)(n_old > 0 ? n_old : 1));
+    int64_t* buf = (int64_t*)malloc(sizeof(int64_t) * (size_t)(n > 0 ? n : 1));
+    if (!idx || !old || !buf) {
+        free(idx); free(old); free(buf);
+        throw_class(env, "java/lang/OutOfMemoryError", "declareCountsRefresh: host buffers");
+        return NULL;
+    }
+    (*env)->GetLongArrayRegion(env, traceIdx, 0, nl, (jlong*)idx);
+    (*env)->GetLongArrayRegion(env, oldCounts, 0, (jsize)n_old, (jlong*)old);
+    double ms = 0;
+    const int rc = siesta_multi_declare_counts_refresh((siesta_multi_log*)(intptr_t)oldLog, (siesta_multi_log*)(intptr_t)newLog, nl ? idx : NULL,
+                                                       (int64_t)nl, (int32_t)kCap, old, buf, &ms);
+    jlongArray out = NULL;
+    if (rc != SIESTA_OK) throw_last(env, "siesta_multi_declare_counts_refresh");
+    else {
+        out = (*env)->NewLongArray(env, (jsize)n);
+        if (out) (*env)->SetLongArrayRegion(env, out, 0, (jsize)n, (const jlong*)buf);
+    }
+    free(idx); free(old); free(buf);
+    return out;
+}
+
 /* long whyNotMatch(long log, int[] pattern, long[] constraints, int uncertainty, int step, int k, long[] cand, int flags):
  * WhyNotMatchSASE.evaluate (model/WhyNotMatch/UsingSase/WhyNotMatchSASE.java:37-55) over the candidate traces of a
  * resident log.  constraints: 5 longs per Constraint (posA, posB, kind SIESTA_WNM_GAP|TIME, method SIESTA_WNM_WITHIN|ATLEAST,

@@ -25,6 +25,7 @@ EXPORTS = [
     "siesta_multi_log_shard", "siesta_multi_detect", "siesta_multi_declare_counts", "siesta_multi_why_not_match",
     "siesta_log_filter_time", "siesta_log_group", "siesta_log_source_events",
     "siesta_log_append", "siesta_log_read", "siesta_multi_log_append", "siesta_index_append", "siesta_index_refresh",
+    "siesta_declare_counts_refresh", "siesta_declare_counts_refresh_device", "siesta_multi_declare_counts_refresh",
 ]
 
 
@@ -75,6 +76,8 @@ def lib():
     L.siesta_declare_counts_size.restype = i64
     L.siesta_declare_counts.argtypes = [vp, i32, vp, P(C.c_double)]
     L.siesta_declare_counts_device.argtypes = [vp, i32, vp, vp, P(C.c_double)]
+    L.siesta_declare_counts_refresh.argtypes = [vp, vp, vp, i64, i32, vp, vp, P(C.c_double)]
+    L.siesta_declare_counts_refresh_device.argtypes = [vp, vp, vp, i64, i32, vp, vp, vp, P(C.c_double)]
     L.siesta_index_load.argtypes = [vp, i32, vp, vp, vp, vp, P(vp)]
     L.siesta_index_build.argtypes = [vp, vp, vp, i32, P(vp)]
     L.siesta_index_append.argtypes = [vp, vp, vp, vp, P(vp), P(C.c_double)]
@@ -119,6 +122,7 @@ def lib():
     L.siesta_multi_log_shard.restype = vp
     L.siesta_multi_detect.argtypes = [vp, P(_abi.Nfa), u32, P(P(_abi.Matches))]
     L.siesta_multi_declare_counts.argtypes = [vp, i32, vp, P(C.c_double)]
+    L.siesta_multi_declare_counts_refresh.argtypes = [vp, vp, vp, i64, i32, vp, vp, P(C.c_double)]
     L.siesta_log_filter_time.argtypes = [vp, i64, i32, i64, i32, P(vp)]
     L.siesta_log_group.argtypes = [vp, vp, vp, i32, vp, i32, P(vp), vp, P(i32)]
     L.siesta_log_source_events.argtypes = [vp, vp]

@@ -219,6 +219,26 @@ class EventLog:
                                                  C.c_void_p(stream) if stream else None, C.byref(ms)))
         return ms.value
 
+    def declare_counts_refresh(self, old_log, old, trace_idx):
+        """siesta_declare_counts_refresh: this log's counts from `old` (DeclareCounts of old_log, or of an earlier
+        refresh) after old_log grew into this log by appends that listed trace_idx (their union, ascending) ->
+        DeclareCounts equal to self.declare_counts(old.k_cap).  Only the listed traces are counted again."""
+        ti, old_packed = _refresh_args(old_log, old, trace_idx)
+        out = np.zeros(lib().siesta_declare_counts_size(self.n_activities, old.k_cap), dtype=np.int64)
+        ms = C.c_double(0.0)
+        check(lib().siesta_declare_counts_refresh(old_log._h, self._h, _ptr(ti) if len(ti) else None, len(ti), int(old.k_cap),
+                                                  _ptr(old_packed), _ptr(out), C.byref(ms)))
+        return _abi.DeclareCounts(out, self.n_activities, old.k_cap, ms.value)
+
+    def declare_counts_refresh_device(self, old_log, d_old, d_out, trace_idx, k_cap, stream=None):
+        """siesta_declare_counts_refresh_device: d_old (packed counts of old_log, CUDA int64 tensor) -> d_out (this log's
+        layout; may be d_old when the alphabet did not grow) -> kernel_ms."""
+        ti = np.ascontiguousarray(trace_idx, dtype=np.int64)
+        ms = C.c_double(0.0)
+        check(lib().siesta_declare_counts_refresh_device(old_log._h, self._h, _ptr(ti) if len(ti) else None, len(ti), int(k_cap),
+                                                         C.c_void_p(d_old.data_ptr()), C.c_void_p(d_out.data_ptr()),
+                                                         C.c_void_p(stream) if stream else None, C.byref(ms)))
+        return ms.value
 
     def pair_stats(self, pairs):
         """siesta_pair_stats: the Count record of each (A,B) pair (kernel K4) -> list of dicts with exact python ints."""
@@ -273,6 +293,13 @@ class EventLog:
     def load_index(self, pairs, lists):
         """siesta_index_load: posting lists (ascending trace indices) produced elsewhere, e.g. index.parquet."""
         return PairIndex(self, pairs, lists=lists)
+
+
+def _refresh_args(old_log, old, trace_idx):
+    """(trace_idx int64, old packed counts) of a count refresh; the counts must be laid out for old_log's alphabet."""
+    if old.n_activities != old_log.n_activities:
+        raise ValueError(f"the old counts are for {old.n_activities} activities, old_log has {old_log.n_activities}")
+    return np.ascontiguousarray(trace_idx, dtype=np.int64), np.ascontiguousarray(old.packed, dtype=np.int64)
 
 
 def _flat_lists(lists):
@@ -480,6 +507,16 @@ class MultiLog:
         ms = C.c_double(0.0)
         check(lib().siesta_multi_declare_counts(self._h, int(k_cap), _ptr(out), C.byref(ms)))
         return _abi.DeclareCounts(out, self.n_activities, int(k_cap), ms.value)
+
+    def declare_counts_refresh(self, old_log, old, trace_idx):
+        """siesta_multi_declare_counts_refresh: EventLog.declare_counts_refresh with GLOBAL trace indices, for this log
+        grown from old_log by MultiLog.append."""
+        ti, old_packed = _refresh_args(old_log, old, trace_idx)
+        out = np.zeros(lib().siesta_declare_counts_size(self.n_activities, old.k_cap), dtype=np.int64)
+        ms = C.c_double(0.0)
+        check(lib().siesta_multi_declare_counts_refresh(old_log._h, self._h, _ptr(ti) if len(ti) else None, len(ti), int(old.k_cap),
+                                                        _ptr(old_packed), _ptr(out), C.byref(ms)))
+        return _abi.DeclareCounts(out, self.n_activities, old.k_cap, ms.value)
 
     def close(self):
         if self._h:

@@ -165,6 +165,28 @@ int validate_act_range(Log* L, int64_t first_event, int64_t n_events, cudaStream
 // Host checks of an appended batch against a log of T traces (siesta_log_append's rules; sets the error, append.cu)
 bool append_check_batch(const char* fn, int64_t T, const int64_t* trace_idx, const int64_t* batch_off, int64_t n_listed,
                         const int32_t* act, const int64_t* ts_ms, int64_t n_new_traces);
+// K3 refresh after a log append on one log (declare.cu; siesta_multi_declare_counts_refresh runs it on every shard)
+struct DeclareRefresh {
+    Log* O = nullptr;                  // the log before the append (only read)
+    Log* N = nullptr;                  // the log after it
+    int64_t n_listed = 0, n_old = 0;   // listed traces; those below O's n_traces (a prefix of the ascending list)
+    int64_t* d_work = nullptr;         // the listed traces on the device (in `block`)
+    int64_t max_old = 0, max_new = 0;  // longest listed trace in O / N (measured for pair-kernel alphabets only)
+    void* block = nullptr;             // arena blocks, returned by declare_refresh_release
+    void* scratch = nullptr;
+};
+// host checks (null trace_idx, k_cap, contexts, derived or blocked logs, shrinking logs, trace_idx; sets the error)
+bool declare_refresh_check_host(const char* fn, const Log* O, const Log* N, const int64_t* trace_idx, int64_t n_listed, int32_t k_cap);
+bool declare_refresh_needs_full(const Log* O, const Log* N);
+// listed traces to the device (`copied`, may be null, is recorded after the copy) + the device check of the unlisted traces'
+// lengths (SIESTA_E_INVALID) + pair widths; waits
+int declare_refresh_stage(const char* fn, DeclareRefresh* r, const int64_t* trace_idx, cudaStream_t stream, cudaEvent_t copied);
+// d_delta (N's layout) = K3(N, listed) - K3(O, listed old traces); enqueues only
+int declare_refresh_delta(DeclareRefresh* r, int32_t k_cap, int64_t* d_delta, cudaStream_t stream);
+// d_out = d_old moved from alphabet A0 to A1 + d_delta (d_out may be d_delta, or d_old when A0 == A1); enqueues only
+int declare_merge(const int64_t* d_old, int32_t A0, int32_t A1, int32_t k_cap, const int64_t* d_delta, int64_t* d_out, const Ctx* c,
+                  cudaStream_t stream);
+void declare_refresh_release(DeclareRefresh* r, cudaStream_t stream);
 int assemble_matches(Ctx* c, std::vector<siesta_dev_matches>& parts, uint32_t flags, cudaStream_t stream, siesta_matches** out,
                      const std::vector<Ctx*>* part_ctx);
 int detect_device_finish_impl(DetectPending* q, siesta_dev_matches* out);

@@ -1300,6 +1300,176 @@ extern "C" int siesta_multi_declare_counts(siesta_multi_log* lh, int32_t k_cap, 
     return SIESTA_OK;
 }
 
+// siesta_declare_counts_refresh over a sharded log: trace_idx is cut at the shard borders as siesta_multi_log_append cuts
+// it (new traces on the last shard); every shard is checked first (no collective runs for a refused call), then every
+// shard computes its delta on its device, one sum all-reduce joins the deltas and rank 0 merges them into the old counts.
+extern "C" int siesta_multi_declare_counts_refresh(siesta_multi_log* old_h, siesta_multi_log* new_h, const int64_t* trace_idx,
+                                                   int64_t n_listed, int32_t k_cap, const int64_t* old_counts, int64_t* out,
+                                                   double* kernel_ms) {
+    static const char* fn = "siesta_multi_declare_counts_refresh";
+    MultiLog* mo = reinterpret_cast<MultiLog*>(old_h);
+    MultiLog* mn = reinterpret_cast<MultiLog*>(new_h);
+    if (!mo || !mn || !old_counts || !out || n_listed < 0 || (n_listed > 0 && !trace_idx)) {
+        set_error(std::string(fn) + ": null argument");
+        return SIESTA_E_INVALID;
+    }
+    const int n = (int)mo->shard.size();
+    if (mn->m != mo->m || (int)mn->shard.size() != n) {
+        set_error(std::string(fn) + ": the two logs are on different contexts");
+        return SIESTA_E_INVALID;
+    }
+    for (int r = 0; r < n; ++r)
+        if (mn->first[(size_t)r] != mo->first[(size_t)r]) {
+            set_error(std::string(fn) + ": new_log is not old_log grown by siesta_multi_log_append");
+            return SIESTA_E_INVALID;
+        }
+    const int64_t T = mo->first[(size_t)n], T2 = mn->first[(size_t)n];
+    if (T2 < T || mn->n_activities < mo->n_activities) {
+        set_error(std::string(fn) + ": new_log has fewer traces or a smaller alphabet than old_log");
+        return SIESTA_E_INVALID;
+    }
+    int64_t n_new = 0;
+    for (int64_t i = 0; i < n_listed; ++i) {
+        if (trace_idx[i] < 0 || trace_idx[i] >= T2 || (i > 0 && trace_idx[i] <= trace_idx[i - 1])) {
+            set_error(std::string(fn) + ": trace_idx must ascend strictly inside [0, new_log's n_traces)");
+            return SIESTA_E_INVALID;
+        }
+        n_new += trace_idx[i] >= T;
+    }
+    if (n_new != T2 - T) {
+        set_error(std::string(fn) + ": trace_idx must list every trace new_log adds (as passed to siesta_multi_log_append)");
+        return SIESTA_E_INVALID;
+    }
+    // listed traces [cut[r], cut[r + 1]) belong to shard r, local indices
+    std::vector<int64_t> cut((size_t)n + 1, n_listed);
+    cut[0] = 0;
+    for (int r = 1; r < n; ++r) cut[(size_t)r] = (int64_t)(std::lower_bound(trace_idx, trace_idx + n_listed, mo->first[(size_t)r]) - trace_idx);
+    std::vector<std::vector<int64_t>> idx((size_t)n);
+    for (int r = 0; r < n; ++r)
+        for (int64_t i = cut[(size_t)r]; i < cut[(size_t)r + 1]; ++i) idx[(size_t)r].push_back(trace_idx[i] - mo->first[(size_t)r]);
+    for (int r = 0; r < n; ++r)
+        if (!declare_refresh_check_host(fn, mo->shard[(size_t)r], mn->shard[(size_t)r], idx[(size_t)r].data(), (int64_t)idx[(size_t)r].size(), k_cap))
+            return SIESTA_E_INVALID;
+    const int32_t A0 = mo->n_activities, A1 = mn->n_activities;
+    if (A1 < 1 || A1 > 4096) {
+        set_error("declare counting: 1 <= n_activities <= 4096 (the eight A x A count matrices of the result)");
+        return SIESTA_E_UNSUPPORTED;
+    }
+    const int64_t len = siesta_declare_counts_size(A1, k_cap), len0 = siesta_declare_counts_size(A0, k_cap);
+    if ((size_t)len * 8 > mo->m->xchg[0]->cap_bytes) {
+        set_error(std::string(fn) + ": count array larger than the exchange region");
+        return SIESTA_E_NOMEM;
+    }
+    // every shard checks its listed traces on its device before any collective
+    std::vector<DeclareRefresh> rr((size_t)n);
+    std::vector<int> rcs((size_t)n, SIESTA_OK);
+    std::vector<std::string> errs((size_t)n);
+    {
+        std::vector<std::thread> th;
+        for (int r = 0; r < n; ++r)
+            th.emplace_back([&, r] {
+                DeclareRefresh& x = rr[(size_t)r];
+                x.O = mo->shard[(size_t)r];
+                x.N = mn->shard[(size_t)r];
+                x.n_listed = (int64_t)idx[(size_t)r].size();
+                if (cudaSetDevice(x.N->ctx->device) != cudaSuccess) {
+                    rcs[(size_t)r] = SIESTA_E_CUDA;
+                    errs[(size_t)r] = std::string(fn) + ": cudaSetDevice";
+                    return;
+                }
+                rcs[(size_t)r] = declare_refresh_stage(fn, &x, idx[(size_t)r].data(), x.N->ctx->stream, nullptr);
+                if (rcs[(size_t)r]) errs[(size_t)r] = siesta_last_error();
+            });
+        for (std::thread& t : th) t.join();
+    }
+    bool full = false;
+    for (int r = 0; r < n; ++r) full |= declare_refresh_needs_full(mo->shard[(size_t)r], mn->shard[(size_t)r]);
+    auto release_all = [&] {
+        for (int r = 0; r < n; ++r) {
+            cudaSetDevice(rr[(size_t)r].N->ctx->device);
+            declare_refresh_release(&rr[(size_t)r], rr[(size_t)r].N->ctx->stream);
+        }
+    };
+    for (int r = 0; r < n; ++r)
+        if (rcs[(size_t)r] != SIESTA_OK) {
+            release_all();
+            set_error(errs[(size_t)r]);
+            return rcs[(size_t)r];
+        }
+    if (full) {   // ids outside the old alphabet that the new one covers: count the new log in full (the header's fallback)
+        release_all();
+        return siesta_multi_declare_counts(new_h, k_cap, out, kernel_ms);
+    }
+    std::vector<double> ms((size_t)n, 0.0);
+    std::vector<std::thread> th;
+    for (int r = 0; r < n; ++r)
+        th.emplace_back([&, r] {
+            DeclareRefresh& x = rr[(size_t)r];
+            Ctx* c = x.N->ctx;
+            cudaSetDevice(c->device);
+            int64_t* d = nullptr;
+            int64_t* d_old = nullptr;
+            cudaEvent_t e0 = nullptr, e1 = nullptr;
+            int rc = SIESTA_OK;
+            if (cudaMallocAsync((void**)&d, (size_t)len * 8, c->stream) != cudaSuccess) {
+                rc = SIESTA_E_NOMEM;
+                errs[(size_t)r] = std::string(fn) + ": cudaMalloc";
+                d = nullptr;
+            }
+            if (rc == SIESTA_OK && (cudaEventCreate(&e0) != cudaSuccess || cudaEventCreate(&e1) != cudaSuccess ||
+                                    cudaEventRecord(e0, c->stream) != cudaSuccess)) {
+                rc = SIESTA_E_CUDA;
+                errs[(size_t)r] = std::string(fn) + ": cudaEvent";
+            }
+            if (rc == SIESTA_OK) rc = declare_refresh_delta(&x, k_cap, d, c->stream);
+            // the collective runs even after a local failure (with zeros), so that the other ranks are not left waiting
+            if (rc != SIESTA_OK && d) cudaMemsetAsync(d, 0, (size_t)len * 8, c->stream);
+            if (rc != SIESTA_OK && errs[(size_t)r].empty()) errs[(size_t)r] = siesta_last_error();
+            int rc2 = d ? siesta_exchange_allreduce_i64(reinterpret_cast<siesta_exchange*>(mo->m->xchg[(size_t)r]), d, len, SIESTA_REDUCE_SUM, c->stream)
+                        : SIESTA_E_NOMEM;
+            if (rc == SIESTA_OK && rc2 != SIESTA_OK) {
+                rc = rc2;
+                errs[(size_t)r] = siesta_last_error();
+            }
+            if (rc == SIESTA_OK && r == 0) {
+                if (cudaMallocAsync((void**)&d_old, (size_t)len0 * 8, c->stream) != cudaSuccess ||
+                    cudaMemcpyAsync(d_old, old_counts, (size_t)len0 * 8, cudaMemcpyHostToDevice, c->stream) != cudaSuccess) {
+                    rc = SIESTA_E_CUDA;
+                    errs[(size_t)r] = std::string(fn) + ": H2D of the old counts";
+                }
+                if (rc == SIESTA_OK) rc = declare_merge(d_old, A0, A1, k_cap, d, d, c, c->stream);
+                if (rc != SIESTA_OK && errs[(size_t)r].empty()) errs[(size_t)r] = siesta_last_error();
+                if (rc == SIESTA_OK && cudaEventRecord(e1, c->stream) != cudaSuccess) rc = SIESTA_E_CUDA;
+                if (rc == SIESTA_OK && (cudaMemcpyAsync(out, d, (size_t)len * 8, cudaMemcpyDeviceToHost, c->stream) != cudaSuccess ||
+                                        cudaStreamSynchronize(c->stream) != cudaSuccess)) {
+                    rc = SIESTA_E_CUDA;
+                    errs[(size_t)r] = std::string(fn) + ": D2H";
+                }
+            } else if (rc == SIESTA_OK && cudaEventRecord(e1, c->stream) != cudaSuccess) {
+                rc = SIESTA_E_CUDA;
+            }
+            float f = 0.f;
+            if (rc == SIESTA_OK && cudaEventSynchronize(e1) == cudaSuccess && cudaEventElapsedTime(&f, e0, e1) == cudaSuccess) ms[(size_t)r] = f;
+            if (d_old) cudaFreeAsync(d_old, c->stream);
+            if (d) cudaFreeAsync(d, c->stream);
+            declare_refresh_release(&x, c->stream);
+            if (e0) cudaEventDestroy(e0);
+            if (e1) cudaEventDestroy(e1);
+            rcs[(size_t)r] = rc;
+        });
+    for (std::thread& t : th) t.join();
+    double worst = 0;
+    for (int r = 0; r < n; ++r) {
+        worst = std::max(worst, ms[(size_t)r]);
+        if (rcs[(size_t)r] != SIESTA_OK) {
+            set_error(errs[(size_t)r]);
+            return rcs[(size_t)r];
+        }
+    }
+    if (kernel_ms) *kernel_ms = worst;
+    return SIESTA_OK;
+}
+
 
 // Why-not-match over a sharded log: the candidates (global trace indices, ascending) are cut at the shard borders, every
 // device evaluates its own (siesta_why_not_match on the shard, wnm.cu), the answers are concatenated in shard order -
